@@ -2,7 +2,7 @@
 """Headline benchmark: converged 2-agent chicane game solves / s (BASELINE.json configs[1]) and the other BASELINE games.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload chicane|curve|agents3|agents4|merge] [--batch B] [--total T]
+                    [--workload chicane|curve|agents3|agents4|merge] [--batch B] [--total T] [--dump-outputs DIR]
 
 A step = one pass of the solver over B synthetic instances per GPU (randomised initial conditions + warm start,
 dgsqp_b200.montecarlo; B = 10 000 for the headline workload).  `value` is measured with the inputs resident in HBM (CUDA
@@ -37,6 +37,7 @@ import time  # noqa: E402
 
 ROOT = pathlib.Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True             # the benchmark leaves the source tree as it found it (it may be read-only)
 
 METRIC = "converged_game_solves_per_sec"
 UNIT = "solves/s"
@@ -47,6 +48,8 @@ MU_VIO = 1e-10                             # deterministic penalty-weight switch
                                            # of every parity fixture; the class default 0 is the literal DGSQP.py:560 rule
 CPU_ARM_BUDGET_S = 200.0                   # wall budget of the whole `--impl reference` run
 CPU_BASELINE_BUDGET_S = 20.0               # wall budget of the cpu_baseline leg inside the GPU arm
+OUTPUT_FIELDS = ("u", "l", "x", "cost", "cond", "num_iters", "status", "qp_solves")   # BatchResult arrays
+DUMP_BUDGET_BYTES = 60 * 10 ** 6           # array data of --dump-outputs: with the .npy headers below 64 MB
 
 
 # ----------------------------------------------------------------------------- workloads
@@ -263,7 +266,14 @@ def main():
     ap.add_argument("--total", type=int, default=0, help="total instances per step sharded over the ranks (strong scaling)")
     ap.add_argument("--cpu-sample", type=int, default=0, help="instances per step of the CPU arms (0 = from the time budget)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write the last step's result arrays (rank 0) to DIR/<cell>_<field>.npy, "
+                         "float64; above 60 MB a fixed seeded sample of the instances")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the GPU arm (--impl ours)")
     # stdout carries exactly one JSON line: NCCL's own prints (version banner, NCCL_DEBUG output) go to stderr
     os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")
     rank = int(os.environ.get("RANK", "0"))
@@ -375,6 +385,8 @@ def main():
         c["status"], c["iters"], c["qps"] = r.status.cpu().numpy(), r.num_iters.cpu().numpy(), r.qp_solves.cpu().numpy()
         c["cond"] = r.cond.cpu().numpy()
         c["diag"] = c["solver"].last_diag(c["B"])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(pathlib.Path(args.dump_outputs), cells)
 
     # end-to-end through the host-buffer C-ABI call (pinned host memory, copies inside the timed region)
     for c in cells:
@@ -475,6 +487,23 @@ def main():
     if dist is not None:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, cells):
+    """The arrays the timed device path returned in its last step, one file per cell and BatchResult field, in float64
+    (integer fields convert exactly).  When all instances exceed DUMP_BUDGET_BYTES, every cell keeps the same fraction of
+    its instances, drawn by default_rng(0) and kept in batch order: the sample depends on the batch size alone, so two
+    builds run with the same arguments dump the same instances."""
+    import numpy as np
+    out_dir.mkdir(parents=True, exist_ok=True)
+    res = [c["res"] for c in cells]
+    row_bytes = [8 * sum(int(np.prod(getattr(r, f).shape[1:])) for f in OUTPUT_FIELDS) for r in res]
+    frac = min(1.0, DUMP_BUDGET_BYTES / sum(rb * c["B"] for rb, c in zip(row_bytes, cells)))
+    for c, r in zip(cells, res):
+        keep = int(frac * c["B"])
+        idx = np.sort(np.random.default_rng(0).choice(c["B"], keep, replace=False)) if keep < c["B"] else slice(None)
+        for f in OUTPUT_FIELDS:
+            np.save(out_dir / f"{c['label']}_{f}.npy", getattr(r, f).cpu().numpy().astype(np.float64)[idx])
 
 
 def cpu_legs(args, cells, cores, np):

@@ -1,4 +1,4 @@
-"""CUDA path vs the 1000-instance oracle fixture: the numbers behind tests/test_gpu_parity.py::test_large_sample_parity_1000."""
+"""CUDA path vs the large-sample oracle fixture: the numbers behind tests/test_gpu_parity.py::test_large_sample_parity."""
 import sys, pathlib
 ROOT = pathlib.Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
@@ -7,7 +7,7 @@ import dgsqp_b200 as dg
 d = dict(np.load(ROOT / "tests/golden/chicane_N25_seed0_stats.npz").items())
 res = dg.DGSQP(dg.chicane_game(), dg.chicane_params(), print_method=None, mu_vio_thresh=1e-10).solve_batch(d["x0"], d["u_ws"])
 same = (res.status == d["status"]) & (res.num_iters == d["num_iters"])
-print(f"identical (status, iters): {int(same.sum())}/1000; identical status: {int((res.status == d['status']).sum())}")
+print(f"identical (status, iters): {int(same.sum())}/{len(same)}; identical status: {int((res.status == d['status']).sum())}")
 for code, name in ((0, "conv_abs_tol"), (1, "conv_rel_tol")):
     m = same & (d["status"] == code)
     err = np.abs(res.u[m] - d["u"][m]).max(axis=1) / np.maximum(1.0, np.abs(d["u"][m]).max(axis=1))

@@ -2,7 +2,7 @@
 """How far is the PRODUCT mode of the oracle (what the CUDA path implements) from the LITERAL reference rules?
 
 The reference cannot run offline (CasADi / OSQP), so the deviations D1-D3 of DESIGN.md are quantified by running the
-oracle itself in literal mode on the 1000-instance chicane fixture (tests/golden/chicane_N25_seed0_stats.npz, whose stored
+oracle itself in literal mode on the large-sample chicane fixture (tests/golden/chicane_N25_seed0_stats.npz, whose stored
 results are the product mode) and counting the instances whose ``(msg, num_iters)`` change:
 
   D1  QP: OSQP restated at its defaults + polish (oracle/osqp_admm.py) instead of the exact KKT point

@@ -1,7 +1,9 @@
 #!/usr/bin/env python3
-"""Large-sample parity fixture: (status, iterations, QP solves, costs) of the CPU oracle on the first COUNT instances of
-the product sampler's 10 k chicane batch (dgsqp_b200.montecarlo.sample_head_to_head, seed 0 -- the batch bench.py runs).
-Inputs are stored with the results so that the fixture does not depend on the sampler's floating-point environment.
+"""Large-sample parity fixture: (status, iterations, QP solves, costs, solutions u) of the CPU oracle on the first COUNT
+instances of the product sampler's 10 k chicane batch (dgsqp_b200.montecarlo.sample_head_to_head, seed 0 -- the batch
+bench.py runs).  Inputs are stored with the results so that the fixture does not depend on the sampler's floating-point
+environment.  u is stored for the converged instances only (NaN rows elsewhere: nothing compares them), which with the
+default COUNT keeps the file under 1 MB.
 
     python tests/golden/make_golden_stats.py [COUNT] [PROCS]
 """
@@ -36,7 +38,7 @@ def work(args):
 
 
 if __name__ == "__main__":
-    count = int(sys.argv[1]) if len(sys.argv) > 1 else 1000
+    count = int(sys.argv[1]) if len(sys.argv) > 1 else 750
     procs = int(sys.argv[2]) if len(sys.argv) > 2 else (os.cpu_count() or 1)
     for k in ("OMP_NUM_THREADS", "OPENBLAS_NUM_THREADS", "MKL_NUM_THREADS"):
         os.environ[k] = "1"
@@ -49,11 +51,13 @@ if __name__ == "__main__":
         out = pool.map(work, [(i, x0[i], u_ws[i]) for i in range(count)], chunksize=4)
     out.sort(key=lambda o: o[0])
     msgs = ["conv_abs_tol", "conv_rel_tol", "max_it", "diverged", "qp_fail", "time_limit"]
-    np.savez_compressed(OUT / "chicane_N25_seed0_stats.npz", x0=x0, u_ws=u_ws,
-                        status=np.array([msgs.index(o[1]) for o in out], dtype=np.int32),
+    status = np.array([msgs.index(o[1]) for o in out], dtype=np.int32)
+    u = np.stack([o[5] for o in out]).astype(np.float64)
+    u[status > 1] = np.nan
+    np.savez_compressed(OUT / "chicane_N25_seed0_stats.npz", x0=x0, u_ws=u_ws, status=status,
                         num_iters=np.array([o[2] for o in out], dtype=np.int32),
                         qp_solves=np.array([o[3] for o in out], dtype=np.int32),
-                        cost=np.stack([o[4] for o in out]), u=np.stack([o[5] for o in out]).astype(np.float64))
+                        cost=np.stack([o[4] for o in out]), u=u)
     (OUT / "chicane_N25_seed0_stats.json").write_text(json.dumps(dict(
         name="chicane_N25_seed0_stats", count=count, seed=0, generator="tests/golden/make_golden_stats.py (CPU oracle)",
         seconds=time.time() - t0, hist={m: sum(o[1] == m for o in out) for m in msgs}), indent=1))

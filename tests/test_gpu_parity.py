@@ -510,19 +510,20 @@ def test_fused_statistics_equal_host_statistics(big_batch):
     assert fused[0] == 3000 and np.array_equal(fused[:15], host[:15])
 
 
-def test_large_sample_parity_1000():
-    """The CUDA path on the first 1000 instances of the bench batch against the oracle's stored results
+def test_large_sample_parity():
+    """The CUDA path on the first 750 instances of the bench batch against the oracle's stored results
     (tests/golden/chicane_N25_seed0_stats.npz): identical (status, iterations) on at least 99 % -- the bar BASELINE.json
-    states (host build of the kernel source: 995 cold start / 997 warm start) -- and KKT-converged equilibria within
-    1e-6 relative (measured: max 2e-7, median 1e-15)."""
+    states (host build of the kernel source on the first 1000: 995 cold start / 997 warm start) -- and KKT-converged
+    equilibria within 1e-6 relative (measured on the first 1000: max 2e-7, median 1e-15)."""
     d = dict(np.load(GOLDEN / "chicane_N25_seed0_stats.npz").items())
+    B = len(d["status"])
     res = dg.DGSQP(dg.chicane_game(), dg.chicane_params(), print_method=None, mu_vio_thresh=1e-10).solve_batch(d["x0"], d["u_ws"])
     same = (res.status == d["status"]) & (res.num_iters == d["num_iters"])
-    print(f"identical (status, iters): {int(same.sum())}/1000; identical status: {int((res.status == d['status']).sum())}")
+    print(f"identical (status, iters): {int(same.sum())}/{B}; identical status: {int((res.status == d['status']).sum())}")
     assert same.mean() >= 0.99 and (res.status == d["status"]).mean() >= 0.99
     # every instance that converged by the KKT test on the same path: inputs and costs to 1e-6, same QP count
     kkt0 = same & (d["status"] == 0)
-    assert kkt0.sum() > 500 and (res.qp_solves[kkt0] == d["qp_solves"][kkt0]).sum() >= kkt0.sum() - 1
+    assert kkt0.sum() > B // 2 and (res.qp_solves[kkt0] == d["qp_solves"][kkt0]).sum() >= kkt0.sum() - 1
     err0 = np.abs(res.u[kkt0] - d["u"][kkt0]).max(axis=1) / np.maximum(1.0, np.abs(d["u"][kkt0]).max(axis=1))
     assert err0.max() < 1e-6
     cerr = np.abs(res.cost[kkt0] - d["cost"][kkt0]).max(axis=1) / np.maximum(1.0, np.abs(d["cost"][kkt0]).max(axis=1))

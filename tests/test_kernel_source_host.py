@@ -253,8 +253,8 @@ def test_kernel_source_under_asan_ubsan():
 
 
 def test_large_sample_fixture_subset():
-    """Kernel source against the 1000-instance oracle fixture (tests/golden/chicane_N25_seed0_stats.npz, the first 1000
-    instances of the batch bench.py runs): a 96-instance slice here, all 1000 on the GPU (test_gpu_parity.py).
+    """Kernel source against the large-sample oracle fixture (tests/golden/chicane_N25_seed0_stats.npz, the first 750
+    instances of the batch bench.py runs): a 96-instance slice here, all of them on the GPU (test_gpu_parity.py).
     Measured over all 1000 with this host build: identical (status, iterations) on 989, identical status on 992; on the
     541 identical KKT-converged instances u agrees to 2.6e-7 and the QP counts are equal; the instances that differ
     are long non-converging paths (max_it / conv_rel_tol flips), where the iteration is chaotic in the last bits."""
