@@ -1,4 +1,5 @@
-// Highway-merge dynamic game on device: rollout, derivatives, constraints and the condensed game-KKT data.
+// Highway-merge dynamic game on device: rollout, derivatives, the lane rows and the costs; the constraint layout and the
+// condensed game-KKT data are shared with the racing games (game_layout.cuh, game_kkt.cuh).
 //
 // Replaces, for the merge scenario of the reference (scripts/DGSQP_merge_monte_carlo.py: three kinematic unicycles under
 // RK3, quadratic goal-tracking costs :253-304, lane half-planes with pw_const-switched ramp normals :40-74,316-318,
@@ -6,10 +7,9 @@
 // DGSQP._evaluate (DGSQP/solvers/DGSQP.py:509-533):
 //   evaluate_dynamics (:598-601), evaluate_jacobian_A/B (:607-612), evaluate_hessian_E/F/G (:621-628),
 //   f_Du_x (:642-650), f_Cxu (:804-821), f_Du_C (:824-826), f_q (:673-676,898-899), f_Q (:679-727,829-934).
-// Same interface as racing_game.cuh (see game.cuh); the solver stack above is shared.  Differences to the racing
-// games: 4 states per agent (x, y, v, psi), the state cost is present at every stage (costates and value-function
-// Hessians of the cost functions pick up a term per stage), no input-rate terms, and the state rows the
-// constraints read are (x, y, v): lane rows n(x)'(p - c) at every stage, v bounds for k >= 1.
+// Differences to the racing games: 4 states per agent (x, y, v, psi), the state cost is present at every stage (costates
+// and value-function Hessians of the cost functions pick up a term per stage), no input-rate terms, and the state rows
+// the constraints read are (x, y, v): lane rows n(x)'(p - c) at every stage, v bounds for k >= 1.
 #pragma once
 #include "cta.cuh"
 #include "model_unicycle_gen.cuh"
@@ -19,11 +19,14 @@
 #define DG_NUA 2
 #define DG_MAX_NQ (DG_NQA * DG_MAX_AGENTS)
 #define DG_MAX_PAIRS 6
-// per-(stage, agent) sizes of the derivative tables: d fd/d[q;u] (4 x 6), packed second derivatives of the outputs
-// x, y (2 x 10) and their costate contraction (10)
-#define DG_AB_SZ 24
+// per-(stage, agent) sizes of the packed second derivatives of the outputs x, y (2 x 10) and their costate
+// contraction (10)
 #define DG_T2_SZ 20
 #define DG_HC_SZ 10
+// constraint rows per (stage, agent): 2 lane rows at every stage, bounds on v
+#define DG_GAME_ROWS 2
+#define DG_GAME_ROWS_N 2
+#define DG_BOUND_STATE 2
 
 // lane row  n(x)'(p - (pt - r n(x))) <= 0,  n(x) = na for x < brk, nb otherwise (CasADi pw_const, merge.py:66-74)
 struct LaneRow { double brk, na[2], nb[2], pt[2]; };
@@ -39,76 +42,14 @@ struct GameDesc {
   LaneRow lane[DG_MAX_AGENTS][2];
 };
 
-struct Dims {
-  int M, N, nq, nu, n, m, P, nc0, nck, ncN, twoN;
-  int ld;        // leading dimension of the n x n work matrices (odd: conflict-free row AND column walks in shared memory)
-  int sens_sz;   // doubles of packed sensitivity rows per agent
+#include "game_layout.cuh"
+
+struct EvalBuf : EvalTables {
+  const GameDesc* G;   // lane normals are needed by the matrix-free G products (set by game_bind)
 };
 
-DG_HD Dims make_dims(int M, int N) {
-  Dims d;
-  d.M = M; d.N = N; d.nq = DG_NQA * M; d.nu = DG_NUA * M; d.n = d.nu * N;
-  d.P = M * (M - 1) / 2;
-  d.nc0 = 6 * M; d.nck = d.P + 8 * M; d.ncN = d.P + 4 * M;
-  d.m = d.nc0 + (N - 1) * d.nck + d.ncN;
-  d.twoN = 2 * N;
-  d.ld = d.n | 1;
-  d.sens_sz = 3 * N * (N + 1);
-  return d;
-}
-
-// ---- constraint row layout (DGSQP.py:730-821): stage major; [shared (k>=1), agent0(lane x2, in-ub, in-lb (k<N),
-//      v-ub, v-lb (k>0)), agent1(...), ...] ----
-enum { K_COLL = 0, K_LANE = 1, K_INUB = 2, K_INLB = 3, K_STUB = 4, K_STLB = 5 };
-
-DG_DEV int row_off(const Dims& D, int k) { return k == 0 ? 0 : D.nc0 + (k - 1) * D.nck; }
-DG_DEV int row_coll(const Dims& D, int k, int p) { return row_off(D, k) + p; }                        // k>=1
-DG_DEV int row_agent(const Dims& D, int k, int a) {
-  return k == 0 ? 6 * a : (k < D.N ? row_off(D, k) + D.P + 8 * a : row_off(D, k) + D.P + 4 * a);
-}
-DG_DEV int row_lane(const Dims& D, int k, int a, int j) { return row_agent(D, k, a) + j; }
-DG_DEV int row_inub(const Dims& D, int k, int a, int c) { return row_agent(D, k, a) + 2 + c; }         // k<N
-DG_DEV int row_inlb(const Dims& D, int k, int a, int c) { return row_agent(D, k, a) + 4 + c; }         // k<N
-DG_DEV int row_stub(const Dims& D, int k, int a) { return row_agent(D, k, a) + (k < D.N ? 6 : 2); }    // k>=1
-DG_DEV int row_stlb(const Dims& D, int k, int a) { return row_agent(D, k, a) + (k < D.N ? 7 : 3); }    // k>=1
-
-DG_DEV void pair_ij(int M, int p, int& i, int& j) {
-  i = 0;
-  int rem = p;
-  while (rem >= M - 1 - i) { rem -= M - 1 - i; ++i; }
-  j = i + 1 + rem;
-}
-
-DG_DEV void decode_row(const Dims& D, int r, int& k, int& kind, int& a, int& b) {
-  int w;
-  if (r < D.nc0) { k = 0; w = r; }
-  else { k = 1 + (r - D.nc0) / D.nck; if (k > D.N) k = D.N; w = r - row_off(D, k); }
-  if (k >= 1) {
-    if (w < D.P) { kind = K_COLL; pair_ij(D.M, w, a, b); return; }
-    w -= D.P;
-  }
-  const int per = k == 0 ? 6 : (k < D.N ? 8 : 4);
-  a = w / per; w -= a * per;
-  if (w < 2) { kind = K_LANE; b = w; return; }
-  if (k < D.N) {
-    if (w < 4) { kind = K_INUB; b = w - 2; }
-    else if (w < 6) { kind = K_INLB; b = w - 4; }
-    else if (w == 6) { kind = K_STUB; b = 2; }
-    else { kind = K_STLB; b = 2; }
-  } else {
-    kind = w == 2 ? K_STUB : K_STLB; b = 2;
-  }
-}
-
-// packed row decode (k | kind << 6 | a << 9 | b << 11), tabulated once per instance (EvalBuf::rowtab)
-DG_DEV int pack_row(const Dims& D, int r) {
-  int k, kind, a, b;
-  decode_row(D, r, k, kind, a, b);
-  return k | (kind << 6) | (a << 9) | (b << 11);
-}
-DG_DEV void unpack_row(int p, int& k, int& kind, int& a, int& b) { k = p & 63; kind = (p >> 6) & 7; a = (p >> 9) & 3; b = (p >> 11) & 7; }
-
-DG_DEV int uidx(const Dims& D, int a, int k, int c) { return a * D.twoN + 2 * k + c; }
+// attaches the game record to the workspace table (after plan_memory)
+DG_HD void game_bind(EvalBuf& E, const GameDesc* G) { E.G = G; }
 
 // active lane normal at longitudinal position px (pw_const: zero derivative)
 DG_DEV void lane_normal(const LaneRow& L, double px, double& n0, double& n1) {
@@ -116,35 +57,6 @@ DG_DEV void lane_normal(const LaneRow& L, double px, double& n0, double& n1) {
   n0 = hi ? L.nb[0] : L.na[0];
   n1 = hi ? L.nb[1] : L.na[1];
 }
-
-// Per-CTA workspace views (same table as racing_game.cuh; sizes per game through DG_AB_SZ / DG_T2_SZ / DG_HC_SZ)
-struct EvalBuf {
-  double* x;     // (N+1)*nq
-  double* AB;    // N*M*24      d fd / d [q;u]  per (k,a)
-  double* T2;    // N*M*20      second derivatives of the outputs x, y per (k,a)
-  double* S;     // M*3N(N+1)   sensitivity rows (x, y, v) of stages 1..N wrt own inputs, packed: row (a,k,r) holds the
-                 //             2k columns of inputs u^a_0..u^a_{k-1} at  a*sens_sz + 3k(k-1) + r*2k
-  double* g;     // m
-  double* q;     // n   [grad_{u^a} J^a]_a
-  double* gtl;   // n   G' l
-  double* cst;   // (M+1)*(N+1)*nq  costates: f<M of J^f, f==M of l'C
-  double* Hc;    // (M+1)*N*M*10    sum_i p_i * T2[i]
-  double* Vbuf;  // 2*(M+1)*nq*nq  DP value-function Hessians of all functions (double buffered)
-  double* Q;     // n*n raw game Hessian (row major)
-  double* Wrow;  // (M+1)*nq*n  running rows of Dxu_Q^f in the Hessian DP, [(f*nq+q)*n + r]
-  double* tmpS;  // M*N*3   state-row products for G v (and the rollout's position increments)
-  double* cf;    // M*N*3   per (a,k) coefficients for G' w
-  double* lbuf;  // m       staged copy of the multipliers the evaluation runs with
-  int* rowtab;   // m       packed row decode (global memory, read-only after game_row_table)
-  const GameDesc* G;   // lane normals are needed by the matrix-free G products (set by game_bind)
-};
-
-// attaches the game record to the workspace table (after plan_memory)
-DG_HD void game_bind(EvalBuf& E, const GameDesc* G) { E.G = G; }
-
-#define DG_SH_EVAL(E) do { DG_ASSUME_SHARED((E).x); DG_ASSUME_SHARED((E).g); DG_ASSUME_SHARED((E).q); DG_ASSUME_SHARED((E).gtl); \
-  DG_ASSUME_SHARED((E).tmpS); DG_ASSUME_SHARED((E).cf); DG_ASSUME_SHARED((E).AB); DG_ASSUME_SHARED((E).cst); DG_ASSUME_SHARED((E).Hc); \
-  DG_ASSUME_SHARED((E).Vbuf); DG_ASSUME_SHARED((E).Wrow); DG_ASSUME_SHARED((E).T2); DG_ASSUME_SHARED((E).S); DG_ASSUME_SHARED((E).lbuf); } while (0)
 
 // x_{k+1} = rk3(x_k, u_k)  (dynamics_models.py:202-212,325-333).  v and psi are running sums of the inputs, so the
 // serial chain over the horizon only carries additions: (1) thread per agent: v_k, psi_k; (2) thread per (k, agent):
@@ -194,256 +106,72 @@ DG_DEVN void game_linearize(Cta& c, const GameDesc& G, const Dims& D_, const dou
     if (second) unicycle_hess(qk, u + uidx(D, a, k, 0), G.veh, E.T2 + t * DG_T2_SZ);
   }
 }
+// ---- hooks of game_kkt.cuh: lane rows, v bounds ----
+// Lane row (k, a, b):  n(x)'(p - (pt - r n(x))) <= 0  for lane b of agent a, n(x) the active normal of lane_normal.  It is
+// linear in the position p = (x, y), so its G row is n0 S_x + n1 S_y; RowCoef holds n of the row.
+struct RowCoef { double n0, n1; };
 
-template <bool SM>
-DG_DEVN void game_row_table(Cta& c, const Dims& D_, int* rowtab) {
-  const Dims D = D_;
-  DG_FOR(r, D.m) rowtab[r] = pack_row(D, r);
-  c.sync();
+DG_DEV double game_state_ub(const GameDesc& G) { return G.v_ub; }
+DG_DEV double game_state_lb(const GameDesc& G) { return G.v_lb; }
+
+DG_DEV double game_row_value(const GameDesc& G, const Dims& D, const double*, const double*, const double* x, int k,
+                             int a, int b) {
+  const LaneRow& L = G.lane[a][b];
+  const double px = x[k * D.nq + a * DG_NQA], py = x[k * D.nq + a * DG_NQA + 1];
+  double n0, n1;
+  lane_normal(L, px, n0, n1);
+  return n0 * (px - (L.pt[0] - G.lane_r * n0)) + n1 * (py - (L.pt[1] - G.lane_r * n1));
 }
 
-// f_Cxu: one thread per row
-template <bool SM>
-DG_DEVN void game_constraints(Cta& c, const GameDesc& G, const Dims& D_, const double* u, const double* up,
-                              const double* x, double* g, const int* DG_RESTRICT rowtab) {
-  const Dims D = D_;
-  DG_ASSUME_SHARED(x); DG_ASSUME_SHARED(g); DG_ASSUME_SHARED(up);
-  DG_FOR(r, D.m) {
-    int k, kind, a, b;
-    unpack_row(rowtab[r], k, kind, a, b);
-    double val;
-    if (kind == K_COLL) {
-      double dx = x[k * D.nq + a * DG_NQA] - x[k * D.nq + b * DG_NQA];
-      double dy = x[k * D.nq + a * DG_NQA + 1] - x[k * D.nq + b * DG_NQA + 1];
-      double rr = G.obs_r[a] + G.obs_r[b];
-      val = rr * rr - (dx * dx + dy * dy);
-    } else if (kind == K_LANE) {
-      const LaneRow& L = G.lane[a][b];
-      const double px = x[k * D.nq + a * DG_NQA], py = x[k * D.nq + a * DG_NQA + 1];
-      double n0, n1;
-      lane_normal(L, px, n0, n1);
-      val = n0 * (px - (L.pt[0] - G.lane_r * n0)) + n1 * (py - (L.pt[1] - G.lane_r * n1));
-    } else if (kind == K_INUB) val = u[uidx(D, a, k, b)] - G.u_ub[b];
-    else if (kind == K_INLB) val = G.u_lb[b] - u[uidx(D, a, k, b)];
-    else if (kind == K_STUB) val = x[k * D.nq + a * DG_NQA + b] - G.v_ub;
-    else val = G.v_lb - x[k * D.nq + a * DG_NQA + b];
-    g[r] = val;
+DG_DEV double game_row_Gv(const Dims& D, const EvalBuf& E, const double*, int k, int a, int b) {
+  double val = 0.0;
+  if (k >= 1) {
+    double n0, n1;
+    lane_normal(E.G->lane[a][b], E.x[k * D.nq + a * DG_NQA], n0, n1);
+    const double* ta = E.tmpS + (a * D.N + (k - 1)) * 3;
+    val = n0 * ta[0] + n1 * ta[1];
+  }
+  return val;
+}
+
+DG_DEV void game_row_prep(const Dims& D, const EvalBuf& E, int k, int kind, int a, int b, RowCoef& rc) {
+  rc.n0 = 0.0; rc.n1 = 0.0;
+  if (kind == K_GAME) lane_normal(E.G->lane[a][b], E.x[k * D.nq + a * DG_NQA], rc.n0, rc.n1);
+}
+
+DG_DEV void game_row_G(const Dims& D, const EvalBuf& E, const RowCoef& rc, int k, int a, int, int ta, int j, int kj, int,
+                       double& val) {
+  if (ta == a && kj < k) {
+    const double* Sk = E.S + sens_off(D, ta, k, 0) + j;
+    val = rc.n0 * Sk[0] + rc.n1 * Sk[2 * k];
   }
 }
 
-// start of packed sensitivity row (a, k, r): k in 1..N, r in {0:x, 1:y, 2:v}; 2k entries
-DG_DEV int sens_off(const Dims& D, int a, int k, int r) { return a * D.sens_sz + 3 * k * (k - 1) + r * 2 * k; }
+// the lane rows read the sensitivities: no sparse row
+DG_DEV bool game_row_sparse(const Dims&, int, int, int, int&, int&) { return false; }
 
-// Sensitivity rows (f_Du_x restricted to x, y, v): thread per input column (a, j).
-template <bool SM>
-DG_DEVN void game_sens(Cta& c, const Dims& D_, const EvalBuf& E_) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  const int twoN = D.twoN;
-  DG_FOR(t, D.M * twoN) {
-    int a = t / twoN, j = t - a * twoN, kj = j >> 1, cc = j & 1;
-    double s4[DG_NQA];
-    const double* AB = E.AB + (kj * D.M + a) * DG_AB_SZ;
-    for (int i = 0; i < DG_NQA; ++i) s4[i] = AB[i * 6 + 4 + cc];
-    for (int k = kj + 1; k <= D.N; ++k) {
-      if (k > kj + 1) {
-        const double* Ak = E.AB + ((k - 1) * D.M + a) * DG_AB_SZ;
-        double t4[DG_NQA];
-        for (int i = 0; i < DG_NQA; ++i) {
-          double acc = 0.0;
-          for (int jj = 0; jj < DG_NQA; ++jj) acc += Ak[i * 6 + jj] * s4[jj];
-          t4[i] = acc;
-        }
-        for (int i = 0; i < DG_NQA; ++i) s4[i] = t4[i];
-      }
-      double* Sk = E.S + sens_off(D, a, k, 0) + j;
-      Sk[0] = s4[0]; Sk[2 * k] = s4[1]; Sk[4 * k] = s4[2];
-    }
+DG_DEV void game_row_coefs(const Dims& D, const EvalBuf& E, const double* w, int k, int a, double& cx, double& cy) {
+  for (int j = 0; j < 2; ++j) {
+    double n0, n1;
+    lane_normal(E.G->lane[a][j], E.x[k * D.nq + a * DG_NQA], n0, n1);
+    const double wl = w[row_game(D, k, a, j)];
+    cx += wl * n0; cy += wl * n1;
   }
 }
 
-template <bool SM>
-DG_DEV double sens_dot(const Dims& D, const EvalBuf& E, int a, int k, int row, const double* va) {
-  const double* DG_RESTRICT Sk = E.S + sens_off(D, a, k, row);
-  double a0 = 0.0, a1 = 0.0;
-  for (int j = 0; j < 2 * k; j += 2) { a0 += Sk[j] * va[j]; a1 += Sk[j + 1] * va[j + 1]; }
-  return a0 + a1;
-}
-
-// y = G v   (v in R^n agent-major, y in R^m).  Two phases with one sync.
-template <bool SM>
-DG_DEVN void game_G_times(Cta& c, const Dims& D_, const EvalBuf& E_, const double* v, double* y) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_; const GameDesc& G = *E.G;
-  c.sync();
-  DG_FOR(t, D.M * D.N * 3) {
-    int a = t / (D.N * 3), rem = t - a * D.N * 3, k1 = rem / 3, row = rem - k1 * 3;
-    E.tmpS[t] = sens_dot<SM>(D, E, a, k1 + 1, row, v + a * D.twoN);
-  }
-  c.sync();
-  DG_FOR(r, D.m) {
-    int k, kind, a, b;
-    unpack_row(E.rowtab[r], k, kind, a, b);
-    double val;
-    if (kind == K_COLL) {
-      double dx = E.x[k * D.nq + a * DG_NQA] - E.x[k * D.nq + b * DG_NQA];
-      double dy = E.x[k * D.nq + a * DG_NQA + 1] - E.x[k * D.nq + b * DG_NQA + 1];
-      const double* ta = E.tmpS + (a * D.N + (k - 1)) * 3;
-      const double* tb = E.tmpS + (b * D.N + (k - 1)) * 3;
-      val = -2.0 * (dx * (ta[0] - tb[0]) + dy * (ta[1] - tb[1]));
-    } else if (kind == K_LANE) {
-      val = 0.0;
-      if (k >= 1) {
-        double n0, n1;
-        lane_normal(G.lane[a][b], E.x[k * D.nq + a * DG_NQA], n0, n1);
-        const double* ta = E.tmpS + (a * D.N + (k - 1)) * 3;
-        val = n0 * ta[0] + n1 * ta[1];
-      }
-    } else if (kind == K_INUB) val = v[uidx(D, a, k, b)];
-    else if (kind == K_INLB) val = -v[uidx(D, a, k, b)];
-    else if (kind == K_STUB) val = E.tmpS[(a * D.N + (k - 1)) * 3 + 2];
-    else val = -E.tmpS[(a * D.N + (k - 1)) * 3 + 2];
-    y[r] = val;
-  }
-  c.sync();
-}
-
-// per (a,k>=1) coefficients of the state rows in  G' w:  cf = [c_x, c_y, c_v]
-template <bool SM>
-DG_DEV void game_state_coefs(Cta& c, const GameDesc& G, const Dims& D, const EvalBuf& E, const double* w, double* cf) {
-  DG_FOR(t, D.M * D.N) {
-    int a = t / D.N, k = t - a * D.N + 1;
-    double cx = 0.0, cy = 0.0;
-    for (int p = 0; p < D.P; ++p) {
-      int i, j;
-      pair_ij(D.M, p, i, j);
-      if (i != a && j != a) continue;
-      double dx = E.x[k * D.nq + i * DG_NQA] - E.x[k * D.nq + j * DG_NQA];
-      double dy = E.x[k * D.nq + i * DG_NQA + 1] - E.x[k * D.nq + j * DG_NQA + 1];
-      double wl = w[row_coll(D, k, p)] * (i == a ? -2.0 : 2.0);
-      cx += wl * dx; cy += wl * dy;
-    }
-    for (int j = 0; j < 2; ++j) {
-      double n0, n1;
-      lane_normal(G.lane[a][j], E.x[k * D.nq + a * DG_NQA], n0, n1);
-      const double wl = w[row_lane(D, k, a, j)];
-      cx += wl * n0; cy += wl * n1;
-    }
-    cf[t * 3] = cx; cf[t * 3 + 1] = cy;
-    cf[t * 3 + 2] = w[row_stub(D, k, a)] - w[row_stlb(D, k, a)];
+DG_DEV void game_row_lx(const GameDesc& G, const Dims& D, const double* x, const double* l, int k, int a, int comp,
+                        double& v) {
+  for (int j = 0; j < 2; ++j) {
+    double n0, n1;
+    lane_normal(G.lane[a][j], x[k * D.nq + a * DG_NQA], n0, n1);
+    v += l[row_game(D, k, a, j)] * (comp == 0 ? n0 : n1);
   }
 }
 
-// input-dependent (sparse) rows of G' w at input (a,k,cc)
-DG_DEV double game_GT_direct(const Dims& D, const double* w, int a, int k, int cc) {
-  return w[row_inub(D, k, a, cc)] - w[row_inlb(D, k, a, cc)];
-}
+// the lane rows do not read the inputs: only the input-bound rows iub / ilb
+DG_DEV double game_row_GT_direct(const Dims&, const double* w, int, int, int, int iub, int ilb) { return w[iub] - w[ilb]; }
 
-// y = G' w  (w in R^m, y in R^n)
-template <bool SM>
-DG_DEVN void game_GT_times(Cta& c, const Dims& D_, const EvalBuf& E_, const double* w, double* y) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_; const GameDesc& G = *E.G;
-  c.sync();
-  game_state_coefs<SM>(c, G, D, E, w, E.cf);
-  c.sync();
-  DG_FOR(t, D.n) {
-    int a = t / D.twoN, j = t - a * D.twoN, kj = j >> 1, cc = j & 1;
-    double acc = game_GT_direct(D, w, a, kj, cc);
-    for (int k = kj + 1; k <= D.N; ++k) {
-      const double* Sk = E.S + sens_off(D, a, k, 0) + j;
-      const double* cf = E.cf + (a * D.N + (k - 1)) * 3;
-      acc += cf[0] * Sk[0] + cf[1] * Sk[2 * k] + cf[2] * Sk[4 * k];
-    }
-    y[t] = acc;
-  }
-  c.sync();
-}
-
-// dense row r of G into out[n] (all threads cooperate)
-template <bool SM>
-DG_DEVN void game_G_row(Cta& c, const Dims& D_, const EvalBuf& E_, int r, double* out) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_; const GameDesc& G = *E.G;
-  int k, kind, a, b;
-  decode_row(D, r, k, kind, a, b);
-  double n0 = 0.0, n1 = 0.0;
-  if (kind == K_LANE) lane_normal(G.lane[a][b], E.x[k * D.nq + a * DG_NQA], n0, n1);
-  DG_FOR(t, D.n) {
-    int ta = t / D.twoN, j = t - ta * D.twoN, kj = j >> 1, cc = j & 1;
-    double val = 0.0;
-    if (kind == K_COLL) {
-      if ((ta == a || ta == b) && kj < k) {
-        double dx = E.x[k * D.nq + a * DG_NQA] - E.x[k * D.nq + b * DG_NQA];
-        double dy = E.x[k * D.nq + a * DG_NQA + 1] - E.x[k * D.nq + b * DG_NQA + 1];
-        const double* Sk = E.S + sens_off(D, ta, k, 0) + j;
-        double sg = ta == a ? -2.0 : 2.0;
-        val = sg * (dx * Sk[0] + dy * Sk[2 * k]);
-      }
-    } else if (kind == K_LANE) {
-      if (ta == a && kj < k) {
-        const double* Sk = E.S + sens_off(D, ta, k, 0) + j;
-        val = n0 * Sk[0] + n1 * Sk[2 * k];
-      }
-    } else if (kind == K_INUB) { if (ta == a && kj == k && cc == b) val = 1.0; }
-    else if (kind == K_INLB) { if (ta == a && kj == k && cc == b) val = -1.0; }
-    else {
-      if (ta == a && kj < k) {
-        double sv = E.S[sens_off(D, ta, k, 2) + j];
-        val = kind == K_STUB ? sv : -sv;
-      }
-    }
-    out[t] = val;
-  }
-  c.sync();
-}
-
-// Rows of G with a single entry +-1 (input bounds): true, and the entry as (input index << 1 | negative) in t1 (t2 = -1);
-// false for the rows that read the sensitivities.  Same entries as game_G_row.
-DG_DEV bool game_G_sparse(const Dims& D, int r, int& t1, int& t2) {
-  int k, kind, a, b;
-  decode_row(D, r, k, kind, a, b);
-  t1 = t2 = -1;
-  if (kind == K_INUB) { t1 = (a * D.twoN + 2 * k + b) << 1; return true; }
-  if (kind == K_INLB) { t1 = ((a * D.twoN + 2 * k + b) << 1) | 1; return true; }
-  return false;
-}
-
-// Rows ids[0..cnt) of G, transposed: out[t * ldo + c] = G[ids[c]][t], t < n (one warp per row, lanes along the inputs; same
-// entries as game_G_row).  No barrier: the caller synchronises.  Used by the blocked warm start of the QP (qp_gi.cuh).
-template <bool SM>
-DG_DEVN void game_G_cols(Cta& c, const Dims& D_, const EvalBuf& E_, const int* ids, int cnt, double* out, int ldo) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_; const GameDesc& G = *E.G;
-  for (int col = c.warp(); col < cnt; col += c.nwarps()) {
-    int k, kind, a, b;
-    decode_row(D, ids[col], k, kind, a, b);
-    double n0 = 0.0, n1 = 0.0;
-    if (kind == K_LANE) lane_normal(G.lane[a][b], E.x[k * D.nq + a * DG_NQA], n0, n1);
-    for (int t = c.lane(); t < D.n; t += c.wsz) {
-      int ta = t / D.twoN, j = t - ta * D.twoN, kj = j >> 1, cc = j & 1;
-      double val = 0.0;
-      if (kind == K_COLL) {
-        if ((ta == a || ta == b) && kj < k) {
-          double dx = E.x[k * D.nq + a * DG_NQA] - E.x[k * D.nq + b * DG_NQA];
-          double dy = E.x[k * D.nq + a * DG_NQA + 1] - E.x[k * D.nq + b * DG_NQA + 1];
-          const double* Sk = E.S + sens_off(D, ta, k, 0) + j;
-          double sg = ta == a ? -2.0 : 2.0;
-          val = sg * (dx * Sk[0] + dy * Sk[2 * k]);
-        }
-      } else if (kind == K_LANE) {
-        if (ta == a && kj < k) {
-          const double* Sk = E.S + sens_off(D, ta, k, 0) + j;
-          val = n0 * Sk[0] + n1 * Sk[2 * k];
-        }
-      } else if (kind == K_INUB) { if (ta == a && kj == k && cc == b) val = 1.0; }
-      else if (kind == K_INLB) { if (ta == a && kj == k && cc == b) val = -1.0; }
-      else {
-        if (ta == a && kj < k) {
-          double sv = E.S[sens_off(D, ta, k, 2) + j];
-          val = kind == K_STUB ? sv : -sv;
-        }
-      }
-      out[t * ldo + col] = val;
-    }
-  }
-}
-
+// ---- hooks of game_kkt.cuh: costs ----
 // stage / terminal state cost of agent f: (k == N ? term_scale : 1) * 1/2 (q^f - goal^f)' diag(w_q) (q^f - goal^f)
 DG_DEV double cost_lx(const GameDesc& G, const Dims& D, const double* x, int f, int k, int idx) {
   int blk = idx / DG_NQA, comp = idx - blk * DG_NQA;
@@ -457,109 +185,23 @@ DG_DEV double cost_lxx(const GameDesc& G, const Dims& D, int f, int k, int i1, i
   if (blk != f) return 0.0;
   return k == D.N ? G.term_scale * G.w_q[comp] : G.w_q[comp];
 }
+DG_DEV double game_term_lx(const GameDesc& G, const Dims& D, const double* x, int f, int idx) { return cost_lx(G, D, x, f, D.N, idx); }
+DG_DEV double game_stage_lx(const GameDesc& G, const Dims& D, const double* x, int f, int k, int idx) { return cost_lx(G, D, x, f, k, idx); }
+DG_DEV double game_term_lxx(const GameDesc& G, const Dims& D, const double*, int f, int i1, int i2) { return cost_lxx(G, D, f, D.N, i1, i2); }
+DG_DEV double game_stage_lxx(const GameDesc& G, const Dims& D, int f, int k, int i1, int i2) { return cost_lxx(G, D, f, k, i1, i2); }
 
-// d(l'C)/dx_k entry idx (state-dependent rows), k>=1
-DG_DEV double con_lx(const GameDesc& G, const Dims& D, const double* x, const double* l, int k, int idx) {
-  int a = idx / DG_NQA, comp = idx - a * DG_NQA;
-  if (comp == 2) return l[row_stub(D, k, a)] - l[row_stlb(D, k, a)];
-  if (comp > 1) return 0.0;
-  double v = 0.0;
-  for (int p = 0; p < D.P; ++p) {
-    int i, j;
-    pair_ij(D.M, p, i, j);
-    if (i != a && j != a) continue;
-    double dd = x[k * D.nq + i * DG_NQA + comp] - x[k * D.nq + j * DG_NQA + comp];
-    v += l[row_coll(D, k, p)] * (i == a ? -2.0 : 2.0) * dd;
-  }
-  for (int j = 0; j < 2; ++j) {
-    double n0, n1;
-    lane_normal(G.lane[a][j], x[k * D.nq + a * DG_NQA], n0, n1);
-    v += l[row_lane(D, k, a, j)] * (comp == 0 ? n0 : n1);
-  }
-  return v;
+// input cost 1/2 w_u u^2 (t = uidx(a, k, cc)): gradient w_u u, second derivative w_u; no coupling between stages.
+// The gradient is read at each sum of game_gradients, so that w_u u + s stays one fused multiply-add per sum.
+struct InputGrad { const double* w; const double* u; };
+DG_DEV InputGrad game_input_grad(const GameDesc& G, const Dims&, const double* u, const double*, int t, int, int, int cc) {
+  return {&G.w_u[cc], &u[t]};
 }
+DG_DEV double input_grad_plus(const InputGrad& g, double s) { return *g.w * *g.u + s; }
+DG_DEV double game_input_hess(const GameDesc& G, const Dims&, int, int cc) { return G.w_u[cc]; }
+DG_DEV void game_input_hess_prev(const GameDesc&, int, double&, double&) {}
 
-// d2(l'C)/dx_k^2 entry (collision rows only: lanes are linear, pw_const has zero derivative), k>=1
-DG_DEV double con_lxx(const Dims& D, const double* l, int k, int i1, int i2) {
-  int a1 = i1 / DG_NQA, c1 = i1 - a1 * DG_NQA, a2 = i2 / DG_NQA, c2 = i2 - a2 * DG_NQA;
-  if (c1 > 1 || c1 != c2) return 0.0;
-  double v = 0.0;
-  for (int p = 0; p < D.P; ++p) {
-    int i, j;
-    pair_ij(D.M, p, i, j);
-    double lp = l[row_coll(D, k, p)];
-    if (a1 == a2) { if (a1 == i || a1 == j) v += -2.0 * lp; }
-    else if ((a1 == i && a2 == j) || (a1 == j && a2 == i)) v += 2.0 * lp;
-  }
-  return v;
-}
-
-// Costate chains  p_k = l_x,k + A_k' p_{k+1}:  thread per (function f, agent block b).
-// f < M: cost of agent f (state cost at every stage); f == M: l'C.
-template <bool SM>
-DG_DEVN void game_costates(Cta& c, const GameDesc& G, const Dims& D_, const EvalBuf& E_, const double* l) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  DG_FOR(t, (D.M + 1) * D.M) {
-    int f = t / D.M, b = t - f * D.M;
-    double p[DG_NQA];
-    double* out = E.cst + f * (D.N + 1) * D.nq;
-    for (int i = 0; i < DG_NQA; ++i) {
-      p[i] = f < D.M ? cost_lx(G, D, E.x, f, D.N, b * DG_NQA + i) : con_lx(G, D, E.x, l, D.N, b * DG_NQA + i);
-      out[D.N * D.nq + b * DG_NQA + i] = p[i];
-    }
-    for (int k = D.N - 1; k >= 0; --k) {
-      const double* Ak = E.AB + (k * D.M + b) * DG_AB_SZ;
-      double pn[DG_NQA];
-      for (int j = 0; j < DG_NQA; ++j) {
-        double acc = 0.0;
-        if (k >= 1) acc = f < D.M ? cost_lx(G, D, E.x, f, k, b * DG_NQA + j) : con_lx(G, D, E.x, l, k, b * DG_NQA + j);
-        for (int i = 0; i < DG_NQA; ++i) acc += Ak[i * 6 + j] * p[i];
-        pn[j] = acc;
-      }
-      for (int i = 0; i < DG_NQA; ++i) { p[i] = pn[i]; out[k * D.nq + b * DG_NQA + i] = pn[i]; }
-    }
-  }
-}
-
-// q (cost gradient, f_q) and G'l from the costates: thread per input (a,k,cc)
-template <bool SM>
-DG_DEVN void game_gradients(Cta& c, const GameDesc& G, const Dims& D_, const EvalBuf& E_, const double* u,
-                            const double* up, const double* l, double* qs) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  DG_FOR(t, D.n) {
-    int a = t / D.twoN, j = t - a * D.twoN, k = j >> 1, cc = j & 1;
-    const double* Bk = E.AB + (k * D.M + a) * DG_AB_SZ;
-    const double* pJ = E.cst + a * (D.N + 1) * D.nq + (k + 1) * D.nq + a * DG_NQA;
-    const double* pC = E.cst + D.M * (D.N + 1) * D.nq + (k + 1) * D.nq + a * DG_NQA;
-    double bj = 0.0, bc = 0.0;
-    for (int i = 0; i < DG_NQA; ++i) { bj += Bk[i * 6 + 4 + cc] * pJ[i]; bc += Bk[i * 6 + 4 + cc] * pC[i]; }
-    E.q[t] = G.w_u[cc] * u[t] + bj;
-    if (qs) {      // grad_u sum_f J^f, only wanted by the v2 merit 'sum_obj_l1' (DGSQP_v2.py:1149-1151)
-      double bs = bj;
-      for (int f = 0; f < D.M; ++f) {
-        if (f == a) continue;
-        const double* pF = E.cst + f * (D.N + 1) * D.nq + (k + 1) * D.nq + a * DG_NQA;
-        for (int i = 0; i < DG_NQA; ++i) bs += Bk[i * 6 + 4 + cc] * pF[i];
-      }
-      qs[t] = G.w_u[cc] * u[t] + bs;
-    }
-    E.gtl[t] = game_GT_direct(D, l, a, k, cc) + bc;
-  }
-}
-
-// Hc[f][k][a][0..9] = sum_{i in {x,y}} p^f_{k+1}[a,i] * T2[k][a][i][:]
-template <bool SM>
-DG_DEVN void game_contract(Cta& c, const Dims& D_, const EvalBuf& E_) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  DG_FOR(t, (D.M + 1) * D.N * D.M * DG_HC_SZ) {
-    int e = t % DG_HC_SZ, r = t / DG_HC_SZ;
-    int a = r % D.M; r /= D.M;
-    int k = r % D.N, f = r / D.N;
-    const double* p = E.cst + f * (D.N + 1) * D.nq + (k + 1) * D.nq + a * DG_NQA;
-    const double* T = E.T2 + (k * D.M + a) * DG_T2_SZ;
-    E.Hc[t] = p[0] * T[e] + p[1] * T[DG_HC_SZ + e];
-  }
-}
+// Hc entry e: only the outputs x, y have second derivatives
+DG_DEV double game_contract_entry(const double* p, const double* T, int e) { return p[0] * T[e] + p[1] * T[DG_HC_SZ + e]; }
 
 DG_DEV int tri4(int r, int cc) { return r * 4 - (r * (r - 1)) / 2 + (cc - r); }
 
@@ -572,121 +214,7 @@ DG_DEV double hc_xx(const double* hc, int i, int j) {
 DG_DEV double hc_ux(const double* hc, int cu, int j) { return j >= 2 ? hc[tri4(j - 2, 2 + cu)] : 0.0; }
 DG_DEV double hc_uu(const double* hc, int c1, int c2) { return c1 <= c2 ? hc[tri4(2 + c1, 2 + c2)] : hc[tri4(2 + c2, 2 + c1)]; }
 
-// Game Hessian Q (f_Q): ONE backward sweep over the stages carrying all M+1 functions (the M costs and l'C);
-// same recursion and work decomposition as racing_game.cuh: game_hessian (DGSQP.py:679-727,829-934).
-template <bool SM>
-DG_DEVN void game_hessian(Cta& c, const GameDesc& G, const Dims& D_, const EvalBuf& E_, const double* DG_RESTRICT l) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  const int n = D.n, nq = D.nq, nu = D.nu, N = D.N, M = D.M, F = D.M + 1;
-  double* Vcur = E.Vbuf;
-  double* Vnext = E.Vbuf + F * nq * nq;
-  double* DG_RESTRICT TV = E.Vbuf + 2 * F * nq * nq;            // [(f*nu + rr)*nq + j]
-  DG_FOR(t, F * nq * nq) {
-    int f = t / (nq * nq), e = t - f * nq * nq, i1 = e / nq, i2 = e - i1 * nq;
-    Vcur[t] = f < M ? cost_lxx(G, D, f, N, i1, i2) : con_lxx(D, l, N, i1, i2);
-  }
-  c.sync();
-  double* DG_RESTRICT Qm = E.Q;
-  for (int k = N - 1; k >= 0; --k) {
-    const int nlater = n - (k + 1) * nu;                          // rows with k_r > k
-    const int nA1 = nlater * M, nA2 = F * nu * nq, nA3 = F * nq * nq;
-    for (int t = c.tid(); t < nA1 + nA2 + nA3; t += c.nt()) {
-      if (t < nA1) {
-        // row r (stage-major input (k_r, a_r, c_r), k_r > k) of Dxu_Q^f through agent block b of stage k
-        const int b = t / nlater, r = (k + 1) * nu + (t - b * nlater);
-        const int kr = r / nu, ar = (r - kr * nu) >> 1, cr = r & 1;
-        const int rowQ = uidx(D, ar, kr, cr);
-        double* DG_RESTRICT wr = E.Wrow + r;                     // w^f[q] at wr[(f*nq + q)*n]
-        const double* DG_RESTRICT ABk = E.AB + (k * M + b) * DG_AB_SZ;
-        double hM0 = 0.0, hM1 = 0.0, hA0 = 0.0, hA1 = 0.0, hB0 = 0.0, hB1 = 0.0;
-        for (int f = 0; f < F; ++f) {
-          double wv[DG_NQA];
-#pragma unroll
-          for (int i = 0; i < DG_NQA; ++i) wv[i] = wr[(f * nq + b * DG_NQA + i) * n];
-          if (f == M || f == ar || f == b) {
-            double v0 = 0.0, v1 = 0.0;
-#pragma unroll
-            for (int i = 0; i < DG_NQA; ++i) { v0 += wv[i] * ABk[i * 6 + 4]; v1 += wv[i] * ABk[i * 6 + 5]; }
-            if (f == M) { hM0 = v0; hM1 = v1; }
-            if (f == ar) { hA0 = v0; hA1 = v1; }
-            if (f == b) { hB0 = v0; hB1 = v1; }
-          }
-#pragma unroll
-          for (int j = 0; j < DG_NQA; ++j) {
-            double acc = 0.0;
-#pragma unroll
-            for (int i = 0; i < DG_NQA; ++i) acc += wv[i] * ABk[i * 6 + j];
-            wr[(f * nq + b * DG_NQA + j) * n] = acc;
-          }
-        }
-        const int colQ = uidx(D, b, k, 0);
-        Qm[rowQ * n + colQ] = hA0 + hM0;  Qm[rowQ * n + colQ + 1] = hA1 + hM1;
-        Qm[colQ * n + rowQ] = hB0 + hM0;  Qm[(colQ + 1) * n + rowQ] = hB1 + hM1;
-      } else if (t < nA1 + nA2) {
-        // tv = B_k' V^f  (row (a_r, c_r), column j)
-        const int e = t - nA1, f = e / (nu * nq), rem = e - f * nu * nq, rr = rem / nq, j = rem - rr * nq;
-        const int ar = rr >> 1, cr = rr & 1;
-        const double* DG_RESTRICT ABa = E.AB + (k * M + ar) * DG_AB_SZ;
-        const double* DG_RESTRICT Vf = Vcur + f * nq * nq;
-        double acc = 0.0;
-#pragma unroll
-        for (int i = 0; i < DG_NQA; ++i) acc += ABa[i * 6 + 4 + cr] * Vf[(ar * DG_NQA + i) * nq + j];
-        TV[e] = acc;
-      } else {
-        // V_k = lxx_k + A'VA + E.p  for every function (into the other buffer)
-        const int tt = t - nA1 - nA2;
-        const int f = tt / (nq * nq), e = tt - f * nq * nq;
-        const int i1 = e / nq, i2 = e - i1 * nq, b1 = i1 / DG_NQA, b2 = i2 / DG_NQA, c1 = i1 - b1 * DG_NQA, c2 = i2 - b2 * DG_NQA;
-        const double* DG_RESTRICT A1 = E.AB + (k * M + b1) * DG_AB_SZ;
-        const double* DG_RESTRICT A2 = E.AB + (k * M + b2) * DG_AB_SZ;
-        const double* DG_RESTRICT Vf = Vcur + f * nq * nq;
-        double acc = f < M ? cost_lxx(G, D, f, k, i1, i2) : (k >= 1 ? con_lxx(D, l, k, i1, i2) : 0.0);
-        if (b1 == b2) acc += hc_xx(E.Hc + ((f * N + k) * M + b1) * DG_HC_SZ, c1, c2);
-#pragma unroll
-        for (int i = 0; i < DG_NQA; ++i) {
-          double rowacc = 0.0;
-#pragma unroll
-          for (int j = 0; j < DG_NQA; ++j) rowacc += Vf[(b1 * DG_NQA + i) * nq + b2 * DG_NQA + j] * A2[j * 6 + c2];
-          acc += A1[i * 6 + c1] * rowacc;
-        }
-        Vnext[tt] = acc;
-      }
-    }
-    c.sync();
-    const int nB1 = F * nu * nq, nB2 = nu * M * 2;
-    for (int t = c.tid(); t < nB1 + nB2; t += c.nt()) {
-      if (t < nB1) {
-        // w = tv A_k + (G.p)[(ar,cr), ar-block]
-        const int f = t / (nu * nq), rem = t - f * nu * nq, rr = rem / nq, q = rem - rr * nq, b = q / DG_NQA, j = q - b * DG_NQA;
-        const int ar = rr >> 1, cr = rr & 1;
-        const double* DG_RESTRICT ABb = E.AB + (k * M + b) * DG_AB_SZ;
-        const double* DG_RESTRICT tv = TV + (f * nu + rr) * nq + b * DG_NQA;
-        double acc = b == ar ? hc_ux(E.Hc + ((f * N + k) * M + ar) * DG_HC_SZ, cr, j) : 0.0;
-#pragma unroll
-        for (int i = 0; i < DG_NQA; ++i) acc += tv[i] * ABb[i * 6 + j];
-        E.Wrow[(f * nq + q) * n + k * nu + rr] = acc;
-      } else {
-        // same-stage block luu + B'VB + F.p  of the functions M and a_r
-        const int e = t - nB1, rr = e / (M * 2), rem = e - rr * M * 2, b = rem >> 1, cc = rem & 1;
-        const int ar = rr >> 1, cr = rr & 1;
-        const double* DG_RESTRICT ABb = E.AB + (k * M + b) * DG_AB_SZ;
-        double vM = 0.0, vA = 0.0;
-        const double* DG_RESTRICT tvM = TV + (M * nu + rr) * nq + b * DG_NQA;
-        const double* DG_RESTRICT tvA = TV + (ar * nu + rr) * nq + b * DG_NQA;
-#pragma unroll
-        for (int i = 0; i < DG_NQA; ++i) { vM += tvM[i] * ABb[i * 6 + 4 + cc]; vA += tvA[i] * ABb[i * 6 + 4 + cc]; }
-        if (b == ar) {
-          vM += hc_uu(E.Hc + ((M * N + k) * M + ar) * DG_HC_SZ, cr, cc);
-          vA += hc_uu(E.Hc + ((ar * N + k) * M + ar) * DG_HC_SZ, cr, cc);
-          if (cc == cr) vA += G.w_u[cc];
-        }
-        Qm[uidx(D, ar, k, cr) * n + uidx(D, b, k, cc)] = vA + vM;
-      }
-    }
-    c.sync();
-    double* tmp = Vcur; Vcur = Vnext; Vnext = tmp;
-  }
-}
+#include "game_kkt.cuh"
 
 // f_J at the solution (DGSQP.py:476-498, 889-893): thread per agent
 template <bool SM>

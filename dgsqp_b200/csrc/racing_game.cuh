@@ -1,12 +1,13 @@
-// Racing dynamic game on device: rollout, derivatives, constraints and the condensed game-KKT data.
+// Racing dynamic game on device: rollout, derivatives, the input-rate rows and the costs; the constraint layout and the
+// condensed game-KKT data are shared with the merge game (game_layout.cuh, game_kkt.cuh).
 //
 // Replaces, for the racing games of the reference (scripts/DGSQP_ALGAMES_monte_carlo_chicane.py,
 // ..._curve.py, DGSQP_monte_carlo_agents.py), the CasADi functions evaluated by
 // DGSQP._evaluate (DGSQP/solvers/DGSQP.py:509-533):
 //   evaluate_dynamics (:598-601), evaluate_jacobian_A/B (:607-612), evaluate_hessian_E/F/G (:621-628),
 //   f_Du_x (:642-650), f_Cxu (:804-821), f_Du_C (:824-826), f_q (:673-676,898-899), f_Q (:679-727,829-934).
-// The constraint Jacobian G is never materialised: it is kept as the sensitivity rows of the states
-// the constraints read (x, y, e_y) and applied matrix-free (G v, G' w, single rows on demand).
+// The state cost is terminal only (progress and competition on s), the inputs carry w_u and input-rate costs w_du, and
+// the constraints read the states x, y, e_y: track bounds on e_y at k >= 1, input-rate rows at k < N.
 #pragma once
 #include "cta.cuh"
 #include "model_bicycle_gen.cuh"
@@ -17,11 +18,13 @@
 #define DG_NUA 2
 #define DG_MAX_NQ (DG_NQA * DG_MAX_AGENTS)
 #define DG_MAX_PAIRS 6
-// per-(stage, agent) sizes of the derivative tables: d fd/d[q;u] (6 x 8), packed second derivatives (6 x 15) and
-// their costate contraction (15)
-#define DG_AB_SZ 48
+// per-(stage, agent) sizes of the packed second derivatives (6 x 15) and their costate contraction (15)
 #define DG_T2_SZ 90
 #define DG_HC_SZ 15
+// constraint rows per (stage, agent): 4 input-rate rows at k < N, track bounds on e_y
+#define DG_GAME_ROWS 4
+#define DG_GAME_ROWS_N 0
+#define DG_BOUND_STATE 5
 
 struct TrackTable {
   int nseg;
@@ -44,77 +47,12 @@ struct GameDesc {
   double obs_r[DG_MAX_AGENTS];
 };
 
-struct Dims {
-  int M, N, nq, nu, n, m, P, nc0, nck, ncN, twoN;
-  int ld;        // leading dimension of the n x n work matrices (odd: conflict-free row AND column walks in shared memory)
-  int sens_sz;   // doubles of packed sensitivity rows per agent
-};
+#include "game_layout.cuh"
 
-DG_HD Dims make_dims(int M, int N) {
-  Dims d;
-  d.M = M; d.N = N; d.nq = DG_NQA * M; d.nu = DG_NUA * M; d.n = d.nu * N;
-  d.P = M * (M - 1) / 2;
-  d.nc0 = 8 * M; d.nck = d.P + 10 * M; d.ncN = d.P + 2 * M;
-  d.m = d.nc0 + (N - 1) * d.nck + d.ncN;
-  d.twoN = 2 * N;
-  d.ld = d.n | 1;
-  d.sens_sz = 3 * N * (N + 1);
-  return d;
-}
+struct EvalBuf : EvalTables {};
 
-// ---- constraint row layout (DGSQP.py:730-821): stage major; [shared, agent0(...), agent1(...)] ----
-enum { K_COLL = 0, K_RATE = 1, K_INUB = 2, K_INLB = 3, K_STUB = 4, K_STLB = 5 };
-
-DG_DEV int row_off(const Dims& D, int k) { return k == 0 ? 0 : D.nc0 + (k - 1) * D.nck; }
-DG_DEV int row_coll(const Dims& D, int k, int p) { return row_off(D, k) + p; }                        // k>=1
-DG_DEV int row_agent(const Dims& D, int k, int a) {
-  return k == 0 ? 8 * a : (k < D.N ? row_off(D, k) + D.P + 10 * a : row_off(D, k) + D.P + 2 * a);
-}
-DG_DEV int row_rate(const Dims& D, int k, int a, int r) { return row_agent(D, k, a) + r; }             // k<N
-DG_DEV int row_inub(const Dims& D, int k, int a, int c) { return row_agent(D, k, a) + 4 + c; }         // k<N
-DG_DEV int row_inlb(const Dims& D, int k, int a, int c) { return row_agent(D, k, a) + 6 + c; }         // k<N
-DG_DEV int row_stub(const Dims& D, int k, int a) { return row_agent(D, k, a) + (k < D.N ? 8 : 0); }    // k>=1
-DG_DEV int row_stlb(const Dims& D, int k, int a) { return row_agent(D, k, a) + (k < D.N ? 9 : 1); }    // k>=1
-
-DG_DEV void pair_ij(int M, int p, int& i, int& j) {
-  i = 0;
-  int rem = p;
-  while (rem >= M - 1 - i) { rem -= M - 1 - i; ++i; }
-  j = i + 1 + rem;
-}
-
-DG_DEV void decode_row(const Dims& D, int r, int& k, int& kind, int& a, int& b) {
-  int w;
-  if (r < D.nc0) { k = 0; w = r; }
-  else { k = 1 + (r - D.nc0) / D.nck; if (k > D.N) k = D.N; w = r - row_off(D, k); }
-  if (k >= 1) {
-    if (w < D.P) { kind = K_COLL; pair_ij(D.M, w, a, b); return; }
-    w -= D.P;
-  }
-  if (k < D.N) {
-    int per = k == 0 ? 8 : 10;
-    a = w / per; w -= a * per;
-    if (w < 4) { kind = K_RATE; b = w; }
-    else if (w < 6) { kind = K_INUB; b = w - 4; }
-    else if (w < 8) { kind = K_INLB; b = w - 6; }
-    else if (w == 8) { kind = K_STUB; b = 5; }
-    else { kind = K_STLB; b = 5; }
-  } else {
-    a = w / 2; w -= a * 2;
-    kind = w == 0 ? K_STUB : K_STLB; b = 5;
-  }
-}
-
-// The row layout only depends on (M, N): the decode (three integer divisions) is tabulated once per instance
-// (EvalBuf::rowtab, packed k | kind << 6 | a << 9 | b << 11) for the loops that walk all m rows.
-DG_DEV int pack_row(const Dims& D, int r) {
-  int k, kind, a, b;
-  decode_row(D, r, k, kind, a, b);
-  return k | (kind << 6) | (a << 9) | (b << 11);
-}
-DG_DEV void unpack_row(int p, int& k, int& kind, int& a, int& b) { k = p & 63; kind = (p >> 6) & 7; a = (p >> 9) & 3; b = (p >> 11) & 7; }
-
-DG_DEV int uidx(const Dims& D, int a, int k, int c) { return a * D.twoN + 2 * k + c; }
+// attaches the game record to the workspace table (after plan_memory); the racing products need no game data
+DG_HD void game_bind(EvalBuf&, const GameDesc*) {}
 
 // ---- track look-ups (radius_arclength_track.py:199-225; CasADi pw_const / pw_lin / fmod) ----
 DG_DEV void track_eval(const TrackTable& T, double s, double& kappa, double& psit, double& dpsit) {
@@ -136,36 +74,6 @@ DG_DEV void track_eval(const TrackTable& T, double s, double& kappa, double& psi
   }
   kappa = kap; psit = ps; dpsit = dp;
 }
-
-// Per-CTA workspace views (global memory unless noted)
-struct EvalBuf {
-  double* x;     // (N+1)*nq
-  double* AB;    // N*M*48      d fd / d [q;u]  per (k,a)
-  double* T2;    // N*M*90      second derivatives per (k,a)
-  double* S;     // M*3N(N+1)   sensitivity rows (x, y, e_y) of stages 1..N wrt own inputs, packed: row (a,k,r) holds the
-                 //             2k columns of inputs u^a_0..u^a_{k-1} at  a*sens_sz + 3k(k-1) + r*2k
-  double* g;     // m
-  double* q;     // n   [grad_{u^a} J^a]_a
-  double* gtl;   // n   G' l
-  double* cst;   // (M+1)*(N+1)*nq  costates: f<M of J^f, f==M of l'C
-  double* Hc;    // (M+1)*N*M*15    sum_i p_i * T2[i]
-  double* Vbuf;  // 2*(M+1)*nq*nq  DP value-function Hessians of all functions (double buffered)
-  double* Q;     // n*n raw game Hessian (row major)
-  double* Wrow;  // (M+1)*nq*n  running rows of Dxu_Q^f in the Hessian DP, [(f*nq+q)*n + r]
-  double* tmpS;  // M*N*3   state-row products for G v
-  double* cf;    // M*N*3   per (a,k) coefficients for G' w
-  double* lbuf;  // m       staged copy of the multipliers the evaluation runs with
-  int* rowtab;   // m       packed row decode (global memory, read-only after game_row_table)
-};
-
-
-// attaches the game record to the workspace table (after plan_memory); the racing products need no game data
-DG_HD void game_bind(EvalBuf&, const GameDesc*) {}
-
-// shared-memory residency hints for the buffer tables (SM instantiation only)
-#define DG_SH_EVAL(E) do { DG_ASSUME_SHARED((E).x); DG_ASSUME_SHARED((E).g); DG_ASSUME_SHARED((E).q); DG_ASSUME_SHARED((E).gtl); \
-  DG_ASSUME_SHARED((E).tmpS); DG_ASSUME_SHARED((E).cf); DG_ASSUME_SHARED((E).AB); DG_ASSUME_SHARED((E).cst); DG_ASSUME_SHARED((E).Hc); \
-  DG_ASSUME_SHARED((E).Vbuf); DG_ASSUME_SHARED((E).Wrow); DG_ASSUME_SHARED((E).T2); DG_ASSUME_SHARED((E).S); DG_ASSUME_SHARED((E).lbuf); } while (0)
 
 // x_{k+1} = x_k + dt f(x_k,u_k)  (explicit Euler of the Frenet bicycle, dynamics_models.py:1030-1070,90-91).
 // Agents are dynamically decoupled and the stage recursion is serial, so only M threads can walk the horizon.  Everything
@@ -225,264 +133,68 @@ DG_DEVN void game_linearize(Cta& c, const GameDesc& G, const Dims& D_, const dou
     double kap, ps, dp;
     track_eval(G.trk, qk[4], kap, ps, dp);
     double sg = qk[2] > 0 ? 1.0 : -1.0;
-    bicycle_jac(qk, u + uidx(D, a, k, 0), G.veh, kap, ps, dp, sg, E.AB + t * 48);
-    if (second) bicycle_hess(qk, u + uidx(D, a, k, 0), G.veh, kap, ps, dp, sg, E.T2 + t * 90);
+    bicycle_jac(qk, u + uidx(D, a, k, 0), G.veh, kap, ps, dp, sg, E.AB + t * DG_AB_SZ);
+    if (second) bicycle_hess(qk, u + uidx(D, a, k, 0), G.veh, kap, ps, dp, sg, E.T2 + t * DG_T2_SZ);
   }
 }
 
-template <bool SM>
-DG_DEVN void game_row_table(Cta& c, const Dims& D_, int* rowtab) {
-  const Dims D = D_;
-  DG_FOR(r, D.m) rowtab[r] = pack_row(D, r);
-  c.sync();
+// ---- hooks of game_kkt.cuh: input-rate rows, track bounds ----
+// Rate row (k, a, b), b = 2 cc + (0: upper, 1: lower):  du - dt rate_ub[cc] <= 0  or  dt rate_lb[cc] - du <= 0  with
+// du = u^a_k[cc] - u^a_{k-1}[cc]  (u^a_{-1} = up, the previous input).  Its G row has the entries +-1 at u_k, u_{k-1}.
+struct RowCoef {};
+
+DG_DEV double game_state_ub(const GameDesc& G) { return G.half_width; }
+DG_DEV double game_state_lb(const GameDesc& G) { return -G.half_width; }
+
+DG_DEV double game_row_value(const GameDesc& G, const Dims& D, const double* u, const double* up, const double*, int k,
+                             int a, int b) {
+  int cc = b >> 1;
+  double uk = u[uidx(D, a, k, cc)];
+  double um = k == 0 ? up[a * DG_NUA + cc] : u[uidx(D, a, k - 1, cc)];
+  double du = uk - um;
+  return (b & 1) == 0 ? du - G.veh.dt * G.rate_ub[cc] : G.veh.dt * G.rate_lb[cc] - du;
 }
 
-// f_Cxu: one thread per row
-template <bool SM>
-DG_DEVN void game_constraints(Cta& c, const GameDesc& G, const Dims& D_, const double* u, const double* up,
-                              const double* x, double* g, const int* DG_RESTRICT rowtab) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const Dims D = D_;
-  DG_ASSUME_SHARED(x); DG_ASSUME_SHARED(g); DG_ASSUME_SHARED(up);
-  DG_FOR(r, D.m) {
-    int k, kind, a, b;
-    unpack_row(rowtab[r], k, kind, a, b);
-    double val;
-    if (kind == K_COLL) {
-      double dx = x[k * D.nq + a * DG_NQA] - x[k * D.nq + b * DG_NQA];
-      double dy = x[k * D.nq + a * DG_NQA + 1] - x[k * D.nq + b * DG_NQA + 1];
-      double rr = G.obs_r[a] + G.obs_r[b];
-      val = rr * rr - (dx * dx + dy * dy);
-    } else if (kind == K_RATE) {
-      int cc = b >> 1;
-      double uk = u[uidx(D, a, k, cc)];
-      double um = k == 0 ? up[a * DG_NUA + cc] : u[uidx(D, a, k - 1, cc)];
-      double du = uk - um;
-      val = (b & 1) == 0 ? du - G.veh.dt * G.rate_ub[cc] : G.veh.dt * G.rate_lb[cc] - du;
-    } else if (kind == K_INUB) val = u[uidx(D, a, k, b)] - G.u_ub[b];
-    else if (kind == K_INLB) val = G.u_lb[b] - u[uidx(D, a, k, b)];
-    else if (kind == K_STUB) val = x[k * D.nq + a * DG_NQA + b] - G.half_width;
-    else val = -G.half_width - x[k * D.nq + a * DG_NQA + b];
-    g[r] = val;
+DG_DEV double game_row_Gv(const Dims& D, const EvalBuf&, const double* v, int k, int a, int b) {
+  int cc = b >> 1;
+  double dv = v[uidx(D, a, k, cc)] - (k > 0 ? v[uidx(D, a, k - 1, cc)] : 0.0);
+  return (b & 1) == 0 ? dv : -dv;
+}
+
+DG_DEV void game_row_prep(const Dims&, const EvalBuf&, int, int, int, int, RowCoef&) {}
+
+DG_DEV void game_row_G(const Dims&, const EvalBuf&, const RowCoef&, int k, int a, int b, int ta, int, int kj, int cc,
+                       double& val) {
+  if (ta == a && cc == (b >> 1)) {
+    double sg = (b & 1) == 0 ? 1.0 : -1.0;
+    if (kj == k) val = sg;
+    else if (kj == k - 1) val = -sg;
   }
 }
 
-// start of packed sensitivity row (a, k, r): k in 1..N, r in {0:x, 1:y, 2:e_y}; 2k entries
-DG_DEV int sens_off(const Dims& D, int a, int k, int r) { return a * D.sens_sz + 3 * k * (k - 1) + r * 2 * k; }
-
-// Sensitivity rows (f_Du_x restricted to x, y, e_y): thread per input column (a, j).
-template <bool SM>
-DG_DEVN void game_sens(Cta& c, const Dims& D_, const EvalBuf& E_) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  const int twoN = D.twoN;
-  DG_FOR(t, D.M * twoN) {
-    int a = t / twoN, j = t - a * twoN, kj = j >> 1, cc = j & 1;
-    double s6[DG_NQA];
-    const double* AB = E.AB + (kj * D.M + a) * 48;
-    for (int i = 0; i < DG_NQA; ++i) s6[i] = AB[i * 8 + 6 + cc];
-    for (int k = kj + 1; k <= D.N; ++k) {
-      if (k > kj + 1) {
-        const double* Ak = E.AB + ((k - 1) * D.M + a) * 48;
-        double t6[DG_NQA];
-        for (int i = 0; i < DG_NQA; ++i) {
-          double acc = 0.0;
-          for (int jj = 0; jj < DG_NQA; ++jj) acc += Ak[i * 8 + jj] * s6[jj];
-          t6[i] = acc;
-        }
-        for (int i = 0; i < DG_NQA; ++i) s6[i] = t6[i];
-      }
-      double* Sk = E.S + sens_off(D, a, k, 0) + j;
-      Sk[0] = s6[0]; Sk[2 * k] = s6[1]; Sk[4 * k] = s6[5];
-    }
-  }
+DG_DEV bool game_row_sparse(const Dims& D, int k, int a, int b, int& t1, int& t2) {
+  const int neg = (b & 1) == 0 ? 0 : 1;
+  t1 = (uidx(D, a, k, b >> 1) << 1) | neg;
+  if (k >= 1) t2 = (uidx(D, a, k - 1, b >> 1) << 1) | (neg ^ 1);
+  return true;
 }
 
-template <bool SM>
-DG_DEV double sens_dot(const Dims& D, const EvalBuf& E, int a, int k, int row, const double* va) {
-  const double* DG_RESTRICT Sk = E.S + sens_off(D, a, k, row);
-  double a0 = 0.0, a1 = 0.0;
-  for (int j = 0; j < 2 * k; j += 2) { a0 += Sk[j] * va[j]; a1 += Sk[j + 1] * va[j + 1]; }
-  return a0 + a1;
-}
+// the rate rows read no state
+DG_DEV void game_row_coefs(const Dims&, const EvalBuf&, const double*, int, int, double&, double&) {}
+DG_DEV void game_row_lx(const GameDesc&, const Dims&, const double*, const double*, int, int, int, double&) {}
 
-// y = G v   (v in R^n agent-major, y in R^m).  Two phases with one sync.
-template <bool SM>
-DG_DEVN void game_G_times(Cta& c, const Dims& D_, const EvalBuf& E_, const double* v, double* y) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  c.sync();
-  DG_FOR(t, D.M * D.N * 3) {
-    int a = t / (D.N * 3), rem = t - a * D.N * 3, k1 = rem / 3, row = rem - k1 * 3;
-    E.tmpS[t] = sens_dot<SM>(D, E, a, k1 + 1, row, v + a * D.twoN);
-  }
-  c.sync();
-  DG_FOR(r, D.m) {
-    int k, kind, a, b;
-    unpack_row(E.rowtab[r], k, kind, a, b);
-    double val;
-    if (kind == K_COLL) {
-      double dx = E.x[k * D.nq + a * DG_NQA] - E.x[k * D.nq + b * DG_NQA];
-      double dy = E.x[k * D.nq + a * DG_NQA + 1] - E.x[k * D.nq + b * DG_NQA + 1];
-      const double* ta = E.tmpS + (a * D.N + (k - 1)) * 3;
-      const double* tb = E.tmpS + (b * D.N + (k - 1)) * 3;
-      val = -2.0 * (dx * (ta[0] - tb[0]) + dy * (ta[1] - tb[1]));
-    } else if (kind == K_RATE) {
-      int cc = b >> 1;
-      double dv = v[uidx(D, a, k, cc)] - (k > 0 ? v[uidx(D, a, k - 1, cc)] : 0.0);
-      val = (b & 1) == 0 ? dv : -dv;
-    } else if (kind == K_INUB) val = v[uidx(D, a, k, b)];
-    else if (kind == K_INLB) val = -v[uidx(D, a, k, b)];
-    else if (kind == K_STUB) val = E.tmpS[(a * D.N + (k - 1)) * 3 + 2];
-    else val = -E.tmpS[(a * D.N + (k - 1)) * 3 + 2];
-    y[r] = val;
-  }
-  c.sync();
-}
-
-// per (a,k>=1) coefficients of the state rows in  G' w:  cf = [c_x, c_y, c_ey]
-template <bool SM>
-DG_DEV void game_state_coefs(Cta& c, const Dims& D, const EvalBuf& E, const double* w, double* cf) {
-  DG_FOR(t, D.M * D.N) {
-    int a = t / D.N, k = t - a * D.N + 1;
-    double cx = 0.0, cy = 0.0;
-    for (int p = 0; p < D.P; ++p) {
-      int i, j;
-      pair_ij(D.M, p, i, j);
-      if (i != a && j != a) continue;
-      double dx = E.x[k * D.nq + i * DG_NQA] - E.x[k * D.nq + j * DG_NQA];
-      double dy = E.x[k * D.nq + i * DG_NQA + 1] - E.x[k * D.nq + j * DG_NQA + 1];
-      double wl = w[row_coll(D, k, p)] * (i == a ? -2.0 : 2.0);
-      cx += wl * dx; cy += wl * dy;
-    }
-    cf[t * 3] = cx; cf[t * 3 + 1] = cy;
-    cf[t * 3 + 2] = w[row_stub(D, k, a)] - w[row_stlb(D, k, a)];
-  }
-}
-
-// input-dependent (sparse) rows of G' w at input (a,k,cc)
-DG_DEV double game_GT_direct(const Dims& D, const double* w, int a, int k, int cc) {
-  double v = w[row_rate(D, k, a, 2 * cc)] - w[row_rate(D, k, a, 2 * cc + 1)];
-  if (k + 1 < D.N) v -= w[row_rate(D, k + 1, a, 2 * cc)] - w[row_rate(D, k + 1, a, 2 * cc + 1)];
-  v += w[row_inub(D, k, a, cc)] - w[row_inlb(D, k, a, cc)];
+// (G' w)[u^a_k[cc]] of the rate rows of stages k and k+1, then of the input-bound rows iub / ilb
+DG_DEV double game_row_GT_direct(const Dims& D, const double* w, int a, int k, int cc, int iub, int ilb) {
+  double v = w[row_game(D, k, a, 2 * cc)] - w[row_game(D, k, a, 2 * cc + 1)];
+  if (k + 1 < D.N) v -= w[row_game(D, k + 1, a, 2 * cc)] - w[row_game(D, k + 1, a, 2 * cc + 1)];
+  v += w[iub] - w[ilb];
   return v;
 }
 
-// y = G' w  (w in R^m, y in R^n)
-template <bool SM>
-DG_DEVN void game_GT_times(Cta& c, const Dims& D_, const EvalBuf& E_, const double* w, double* y) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  c.sync();
-  game_state_coefs<SM>(c, D, E, w, E.cf);
-  c.sync();
-  DG_FOR(t, D.n) {
-    int a = t / D.twoN, j = t - a * D.twoN, kj = j >> 1, cc = j & 1;
-    double acc = game_GT_direct(D, w, a, kj, cc);
-    for (int k = kj + 1; k <= D.N; ++k) {
-      const double* Sk = E.S + sens_off(D, a, k, 0) + j;
-      const double* cf = E.cf + (a * D.N + (k - 1)) * 3;
-      acc += cf[0] * Sk[0] + cf[1] * Sk[2 * k] + cf[2] * Sk[4 * k];
-    }
-    y[t] = acc;
-  }
-  c.sync();
-}
-
-// dense row r of G into out[n] (all threads cooperate)
-template <bool SM>
-DG_DEVN void game_G_row(Cta& c, const Dims& D_, const EvalBuf& E_, int r, double* out) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  int k, kind, a, b;
-  decode_row(D, r, k, kind, a, b);
-  DG_FOR(t, D.n) {
-    int ta = t / D.twoN, j = t - ta * D.twoN, kj = j >> 1, cc = j & 1;
-    double val = 0.0;
-    if (kind == K_COLL) {
-      if ((ta == a || ta == b) && kj < k) {
-        double dx = E.x[k * D.nq + a * DG_NQA] - E.x[k * D.nq + b * DG_NQA];
-        double dy = E.x[k * D.nq + a * DG_NQA + 1] - E.x[k * D.nq + b * DG_NQA + 1];
-        const double* Sk = E.S + sens_off(D, ta, k, 0) + j;
-        double sg = ta == a ? -2.0 : 2.0;
-        val = sg * (dx * Sk[0] + dy * Sk[2 * k]);
-      }
-    } else if (kind == K_RATE) {
-      if (ta == a && cc == (b >> 1)) {
-        double sg = (b & 1) == 0 ? 1.0 : -1.0;
-        if (kj == k) val = sg;
-        else if (kj == k - 1) val = -sg;
-      }
-    } else if (kind == K_INUB) { if (ta == a && kj == k && cc == b) val = 1.0; }
-    else if (kind == K_INLB) { if (ta == a && kj == k && cc == b) val = -1.0; }
-    else {
-      if (ta == a && kj < k) {
-        double sv = E.S[sens_off(D, ta, k, 2) + j];
-        val = kind == K_STUB ? sv : -sv;
-      }
-    }
-    out[t] = val;
-  }
-  c.sync();
-}
-
-// Rows of G with one or two entries +-1 (input bounds, rate limits): true, and the entries as (input index << 1 | negative)
-// in t1 / t2 (-1 = none); false for the rows that read the sensitivities.  Same entries as game_G_row.
-DG_DEV bool game_G_sparse(const Dims& D, int r, int& t1, int& t2) {
-  int k, kind, a, b;
-  decode_row(D, r, k, kind, a, b);
-  t1 = t2 = -1;
-  if (kind == K_INUB) { t1 = uidx(D, a, k, b) << 1; return true; }
-  if (kind == K_INLB) { t1 = (uidx(D, a, k, b) << 1) | 1; return true; }
-  if (kind == K_RATE) {
-    const int neg = (b & 1) == 0 ? 0 : 1;
-    t1 = (uidx(D, a, k, b >> 1) << 1) | neg;
-    if (k >= 1) t2 = (uidx(D, a, k - 1, b >> 1) << 1) | (neg ^ 1);
-    return true;
-  }
-  return false;
-}
-
-// Rows ids[0..cnt) of G, transposed: out[t * ldo + c] = G[ids[c]][t], t < n (one warp per row, lanes along the inputs; same
-// entries as game_G_row).  No barrier: the caller synchronises.  Used by the blocked warm start of the QP (qp_gi.cuh).
-template <bool SM>
-DG_DEVN void game_G_cols(Cta& c, const Dims& D_, const EvalBuf& E_, const int* ids, int cnt, double* out, int ldo) {
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  for (int col = c.warp(); col < cnt; col += c.nwarps()) {
-    int k, kind, a, b;
-    decode_row(D, ids[col], k, kind, a, b);
-    for (int t = c.lane(); t < D.n; t += c.wsz) {
-      int ta = t / D.twoN, j = t - ta * D.twoN, kj = j >> 1, cc = j & 1;
-      double val = 0.0;
-      if (kind == K_COLL) {
-        if ((ta == a || ta == b) && kj < k) {
-          double dx = E.x[k * D.nq + a * DG_NQA] - E.x[k * D.nq + b * DG_NQA];
-          double dy = E.x[k * D.nq + a * DG_NQA + 1] - E.x[k * D.nq + b * DG_NQA + 1];
-          const double* Sk = E.S + sens_off(D, ta, k, 0) + j;
-          double sg = ta == a ? -2.0 : 2.0;
-          val = sg * (dx * Sk[0] + dy * Sk[2 * k]);
-        }
-      } else if (kind == K_RATE) {
-        if (ta == a && cc == (b >> 1)) {
-          double sg = (b & 1) == 0 ? 1.0 : -1.0;
-          if (kj == k) val = sg;
-          else if (kj == k - 1) val = -sg;
-        }
-      } else if (kind == K_INUB) { if (ta == a && kj == k && cc == b) val = 1.0; }
-      else if (kind == K_INLB) { if (ta == a && kj == k && cc == b) val = -1.0; }
-      else {
-        if (ta == a && kj < k) {
-          double sv = E.S[sens_off(D, ta, k, 2) + j];
-          val = kind == K_STUB ? sv : -sv;
-        }
-      }
-      out[t * ldo + col] = val;
-    }
-  }
-}
-
+// ---- hooks of game_kkt.cuh: costs ----
 // terminal-cost gradient entries of agent f wrt joint x_N:  -c_prog*s_f + sum_b c_comp*atan(s_b - s_f)
-DG_DEV double term_grad(const GameDesc& G, const Dims& D, const double* xN, int f, int idx) {
+DG_DEV double game_term_lx(const GameDesc& G, const Dims& D, const double* x, int f, int idx) {
+  const double* xN = x + D.N * D.nq;
   int blk = idx / DG_NQA, comp = idx - blk * DG_NQA;
   if (comp != 4) return 0.0;
   double sf = xN[f * DG_NQA + 4];
@@ -495,7 +207,8 @@ DG_DEV double term_grad(const GameDesc& G, const Dims& D, const double* xN, int 
   return G.c_comp / (1.0 + dd * dd);
 }
 
-DG_DEV double term_hess(const GameDesc& G, const Dims& D, const double* xN, int f, int i1, int i2) {
+DG_DEV double game_term_lxx(const GameDesc& G, const Dims& D, const double* x, int f, int i1, int i2) {
+  const double* xN = x + D.N * D.nq;
   int b1 = i1 / DG_NQA, c1 = i1 - b1 * DG_NQA, b2 = i2 / DG_NQA, c2 = i2 - b2 * DG_NQA;
   if (c1 != 4 || c2 != 4) return 0.0;
   double sf = xN[f * DG_NQA + 4];
@@ -512,112 +225,36 @@ DG_DEV double term_hess(const GameDesc& G, const Dims& D, const double* xN, int 
   return v;
 }
 
-// d(l'C)/dx_k entry idx (state-dependent rows), k>=1
-DG_DEV double con_lx(const Dims& D, const double* x, const double* l, int k, int idx) {
-  int a = idx / DG_NQA, comp = idx - a * DG_NQA;
-  if (comp == 5) return l[row_stub(D, k, a)] - l[row_stlb(D, k, a)];
-  if (comp > 1) return 0.0;
-  double v = 0.0;
-  for (int p = 0; p < D.P; ++p) {
-    int i, j;
-    pair_ij(D.M, p, i, j);
-    if (i != a && j != a) continue;
-    double dd = x[k * D.nq + i * DG_NQA + comp] - x[k * D.nq + j * DG_NQA + comp];
-    v += l[row_coll(D, k, p)] * (i == a ? -2.0 : 2.0) * dd;
-  }
-  return v;
+// no state cost before the terminal stage
+DG_DEV double game_stage_lx(const GameDesc&, const Dims&, const double*, int, int, int) { return 0.0; }
+DG_DEV double game_stage_lxx(const GameDesc&, const Dims&, int, int, int, int) { return 0.0; }
+
+// d/du^a_k[cc] of the input costs 1/2 w_u u_k^2 + 1/2 w_du (u_k - u_{k-1})^2 of agent a (t = uidx(a, k, cc)), evaluated
+// once and added to each sum of game_gradients
+struct InputGrad { double v; };
+DG_DEV InputGrad game_input_grad(const GameDesc& G, const Dims& D, const double* u, const double* up, int t, int a, int k,
+                                 int cc) {
+  double uk = u[t];
+  double um = k == 0 ? up[a * DG_NUA + cc] : u[t - 2];
+  double val = G.w_u[cc] * uk + G.w_du[cc] * (uk - um);
+  if (k + 1 < D.N) val -= G.w_du[cc] * (u[t + 2] - uk);
+  return {val};
+}
+DG_DEV double input_grad_plus(const InputGrad& g, double s) { return g.v + s; }
+
+// their second derivatives: d2/du_k[cc]^2, and -w_du between u_k and u_{k-1} (added to v0 / v1 for cr = 0 / 1)
+DG_DEV double game_input_hess(const GameDesc& G, const Dims& D, int k, int cc) {
+  return G.w_u[cc] + G.w_du[cc] + (k + 1 < D.N ? G.w_du[cc] : 0.0);
+}
+DG_DEV void game_input_hess_prev(const GameDesc& G, int cr, double& v0, double& v1) {
+  if (cr == 0) v0 -= G.w_du[0]; else v1 -= G.w_du[1];
 }
 
-// d2(l'C)/dx_k^2 entry (collision rows only), k>=1
-DG_DEV double con_lxx(const Dims& D, const double* l, int k, int i1, int i2) {
-  int a1 = i1 / DG_NQA, c1 = i1 - a1 * DG_NQA, a2 = i2 / DG_NQA, c2 = i2 - a2 * DG_NQA;
-  if (c1 > 1 || c1 != c2) return 0.0;
-  double v = 0.0;
-  for (int p = 0; p < D.P; ++p) {
-    int i, j;
-    pair_ij(D.M, p, i, j);
-    double lp = l[row_coll(D, k, p)];
-    if (a1 == a2) { if (a1 == i || a1 == j) v += -2.0 * lp; }
-    else if ((a1 == i && a2 == j) || (a1 == j && a2 == i)) v += 2.0 * lp;
-  }
-  return v;
-}
-
-// Costate chains  p_k = l_x,k + A_k' p_{k+1}:  thread per (function f, agent block b).
-// f < M: cost of agent f (state cost only at the terminal stage); f == M: l'C.
-template <bool SM>
-DG_DEVN void game_costates(Cta& c, const GameDesc& G, const Dims& D_, const EvalBuf& E_, const double* l) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  DG_FOR(t, (D.M + 1) * D.M) {
-    int f = t / D.M, b = t - f * D.M;
-    double p[DG_NQA];
-    double* out = E.cst + f * (D.N + 1) * D.nq;
-    const double* xN = E.x + D.N * D.nq;
-    for (int i = 0; i < DG_NQA; ++i) {
-      p[i] = f < D.M ? term_grad(G, D, xN, f, b * DG_NQA + i) : con_lx(D, E.x, l, D.N, b * DG_NQA + i);
-      out[D.N * D.nq + b * DG_NQA + i] = p[i];
-    }
-    for (int k = D.N - 1; k >= 0; --k) {
-      const double* Ak = E.AB + (k * D.M + b) * 48;
-      double pn[DG_NQA];
-      for (int j = 0; j < DG_NQA; ++j) {
-        double acc = (f == D.M && k >= 1) ? con_lx(D, E.x, l, k, b * DG_NQA + j) : 0.0;
-        for (int i = 0; i < DG_NQA; ++i) acc += Ak[i * 8 + j] * p[i];
-        pn[j] = acc;
-      }
-      for (int i = 0; i < DG_NQA; ++i) { p[i] = pn[i]; out[k * D.nq + b * DG_NQA + i] = pn[i]; }
-    }
-  }
-}
-
-// q (cost gradient, f_q) and G'l from the costates: thread per input (a,k,cc)
-template <bool SM>
-DG_DEVN void game_gradients(Cta& c, const GameDesc& G, const Dims& D_, const EvalBuf& E_, const double* u,
-                            const double* up, const double* l, double* qs) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  DG_FOR(t, D.n) {
-    int a = t / D.twoN, j = t - a * D.twoN, k = j >> 1, cc = j & 1;
-    const double* Bk = E.AB + (k * D.M + a) * 48;
-    const double* pJ = E.cst + a * (D.N + 1) * D.nq + (k + 1) * D.nq + a * DG_NQA;
-    const double* pC = E.cst + D.M * (D.N + 1) * D.nq + (k + 1) * D.nq + a * DG_NQA;
-    double bj = 0.0, bc = 0.0;
-    for (int i = 0; i < DG_NQA; ++i) { bj += Bk[i * 8 + 6 + cc] * pJ[i]; bc += Bk[i * 8 + 6 + cc] * pC[i]; }
-    double uk = u[t];
-    double um = k == 0 ? up[a * DG_NUA + cc] : u[t - 2];
-    double val = G.w_u[cc] * uk + G.w_du[cc] * (uk - um);
-    if (k + 1 < D.N) val -= G.w_du[cc] * (u[t + 2] - uk);
-    E.q[t] = val + bj;
-    if (qs) {      // grad_u sum_f J^f, only wanted by the v2 merit 'sum_obj_l1' (DGSQP_v2.py:1149-1151)
-      // every agent's terminal cost reaches u^a through the states: sum over the cost costates of all functions
-      double bs = bj;
-      for (int f = 0; f < D.M; ++f) {
-        if (f == a) continue;
-        const double* pF = E.cst + f * (D.N + 1) * D.nq + (k + 1) * D.nq + a * DG_NQA;
-        for (int i = 0; i < DG_NQA; ++i) bs += Bk[i * 8 + 6 + cc] * pF[i];
-      }
-      qs[t] = val + bs;
-    }
-    E.gtl[t] = game_GT_direct(D, l, a, k, cc) + bc;
-  }
-}
-
-// Hc[f][k][a][0..14] = sum_i p^f_{k+1}[a,i] * T2[k][a][i][:]
-template <bool SM>
-DG_DEVN void game_contract(Cta& c, const Dims& D_, const EvalBuf& E_) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  DG_FOR(t, (D.M + 1) * D.N * D.M * 15) {
-    int e = t % 15, r = t / 15;
-    int a = r % D.M; r /= D.M;
-    int k = r % D.N, f = r / D.N;
-    const double* p = E.cst + f * (D.N + 1) * D.nq + (k + 1) * D.nq + a * DG_NQA;
-    const double* T = E.T2 + (k * D.M + a) * 90;
-    double acc = 0.0;
-    for (int i = 0; i < DG_NQA; ++i) acc += p[i] * T[i * 15 + e];
-    E.Hc[t] = acc;
-  }
+// Hc entry e: sum over all six states of p_i * T2[i][e]
+DG_DEV double game_contract_entry(const double* p, const double* T, int e) {
+  double acc = 0.0;
+  for (int i = 0; i < DG_NQA; ++i) acc += p[i] * T[i * DG_HC_SZ + e];
+  return acc;
 }
 
 DG_DEV int tri5(int r, int cc) { return r * 5 - (r * (r - 1)) / 2 + (cc - r); }
@@ -631,131 +268,7 @@ DG_DEV double hc_xx(const double* hc, int i, int j) {
 DG_DEV double hc_ux(const double* hc, int cu, int j) { return (cu == 1 && j >= 2) ? hc[tri5(j - 2, 4)] : 0.0; }
 DG_DEV double hc_uu(const double* hc, int c1, int c2) { return (c1 == 1 && c2 == 1) ? hc[14] : 0.0; }
 
-// Game Hessian Q (f_Q): ONE backward sweep over the stages carrying all M+1 functions (the M costs and
-// l'C).   row block a of Q = grad_{u^a} grad_u (J^a + l'C)   (DGSQP.py:920-934)
-// Row r (stage-major input index (k_r, a_r, c_r)) of Dxu_Q^f is kept as w^f in E.Wrow[(f*nq + q)*n + r] for every
-// function f.  At stage k < k_r the row emits H^f[r, (k,b,cc)] = w^f[b] . B^b_k[:,cc] and
-// Q[r][(k,b,cc)] = H^{a_r} + H^M  and, by symmetry of each H^f,  Q[(k,b,cc)][r] = H^b + H^M.
-// Every entry of Q is written exactly once, so Q needs no zero-fill and no read-modify-write.
-// Per stage, two barrier intervals whose work items are spread over the whole CTA:
-//   A: (row r with k_r > k, agent block b): propagate w through A_k^b and emit the two Q entries       [n_later*M items]
-//      (function f, new row (a_r,c_r), column j): tv = B_k' V^f  (first half of the same-stage products) [F*nu*nq items]
-//      (function f, i1, i2): V_k = lxx_k + A'VA + E.p                                                      [F*nq*nq items]
-//   B: (f, new row, b, j): w = tv A_k + (G.p)   and   (new row, b, cc): same-stage block luu + B'VB + F.p
-template <bool SM>
-DG_DEVN void game_hessian(Cta& c, const GameDesc& G, const Dims& D_, const EvalBuf& E_, const double* DG_RESTRICT l) {
-  // local copies: the tables live in shared memory and would otherwise be re-read after every store
-  const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  const int n = D.n, nq = D.nq, nu = D.nu, N = D.N, M = D.M, F = D.M + 1;
-  const double* xN = E.x + N * nq;
-  double* Vcur = E.Vbuf;
-  double* Vnext = E.Vbuf + F * nq * nq;
-  double* DG_RESTRICT TV = E.Vbuf + 2 * F * nq * nq;            // [(f*nu + rr)*nq + j]
-  DG_FOR(t, F * nq * nq) {
-    int f = t / (nq * nq), e = t - f * nq * nq, i1 = e / nq, i2 = e - i1 * nq;
-    Vcur[t] = f < M ? term_hess(G, D, xN, f, i1, i2) : con_lxx(D, l, N, i1, i2);
-  }
-  c.sync();
-  double* DG_RESTRICT Qm = E.Q;
-  for (int k = N - 1; k >= 0; --k) {
-    const int nlater = n - (k + 1) * nu;                          // rows with k_r > k
-    const int nA1 = nlater * M, nA2 = F * nu * nq, nA3 = F * nq * nq;
-    for (int t = c.tid(); t < nA1 + nA2 + nA3; t += c.nt()) {
-      if (t < nA1) {
-        const int b = t / nlater, r = (k + 1) * nu + (t - b * nlater);
-        const int kr = r / nu, ar = (r - kr * nu) >> 1, cr = r & 1;
-        const int rowQ = uidx(D, ar, kr, cr);
-        double* DG_RESTRICT wr = E.Wrow + r;                     // w^f[q] at wr[(f*nq + q)*n]
-        const double* DG_RESTRICT ABk = E.AB + (k * M + b) * 48;
-        double hM0 = 0.0, hM1 = 0.0, hA0 = 0.0, hA1 = 0.0, hB0 = 0.0, hB1 = 0.0;
-        for (int f = 0; f < F; ++f) {
-          double wv6[DG_NQA];
-#pragma unroll
-          for (int i = 0; i < DG_NQA; ++i) wv6[i] = wr[(f * nq + b * DG_NQA + i) * n];
-          if (f == M || f == ar || f == b) {
-            double v0 = 0.0, v1 = 0.0;
-#pragma unroll
-            for (int i = 0; i < DG_NQA; ++i) { v0 += wv6[i] * ABk[i * 8 + 6]; v1 += wv6[i] * ABk[i * 8 + 7]; }
-            if (f < M && kr == k + 1 && b == ar && f == ar) { if (cr == 0) v0 -= G.w_du[0]; else v1 -= G.w_du[1]; }
-            if (f == M) { hM0 = v0; hM1 = v1; }
-            if (f == ar) { hA0 = v0; hA1 = v1; }
-            if (f == b) { hB0 = v0; hB1 = v1; }
-          }
-#pragma unroll
-          for (int j = 0; j < DG_NQA; ++j) {
-            double acc = 0.0;
-#pragma unroll
-            for (int i = 0; i < DG_NQA; ++i) acc += wv6[i] * ABk[i * 8 + j];
-            wr[(f * nq + b * DG_NQA + j) * n] = acc;
-          }
-        }
-        const int colQ = uidx(D, b, k, 0);
-        Qm[rowQ * n + colQ] = hA0 + hM0;  Qm[rowQ * n + colQ + 1] = hA1 + hM1;
-        Qm[colQ * n + rowQ] = hB0 + hM0;  Qm[(colQ + 1) * n + rowQ] = hB1 + hM1;
-      } else if (t < nA1 + nA2) {
-        const int e = t - nA1, f = e / (nu * nq), rem = e - f * nu * nq, rr = rem / nq, j = rem - rr * nq;
-        const int ar = rr >> 1, cr = rr & 1;
-        const double* DG_RESTRICT ABa = E.AB + (k * M + ar) * 48;
-        const double* DG_RESTRICT Vf = Vcur + f * nq * nq;
-        double acc = 0.0;
-#pragma unroll
-        for (int i = 0; i < DG_NQA; ++i) acc += ABa[i * 8 + 6 + cr] * Vf[(ar * DG_NQA + i) * nq + j];
-        TV[e] = acc;
-      } else {
-        // V_k = lxx_k + A'VA + E.p  for every function (into the other buffer)
-        const int tt = t - nA1 - nA2;
-        const int f = tt / (nq * nq), e = tt - f * nq * nq;
-        const int i1 = e / nq, i2 = e - i1 * nq, b1 = i1 / DG_NQA, b2 = i2 / DG_NQA, c1 = i1 - b1 * DG_NQA, c2 = i2 - b2 * DG_NQA;
-        const double* DG_RESTRICT A1 = E.AB + (k * M + b1) * 48;
-        const double* DG_RESTRICT A2 = E.AB + (k * M + b2) * 48;
-        const double* DG_RESTRICT Vf = Vcur + f * nq * nq;
-        double acc = (f == M && k >= 1) ? con_lxx(D, l, k, i1, i2) : 0.0;
-        if (b1 == b2) acc += hc_xx(E.Hc + ((f * N + k) * M + b1) * 15, c1, c2);
-#pragma unroll
-        for (int i = 0; i < DG_NQA; ++i) {
-          double rowacc = 0.0;
-#pragma unroll
-          for (int j = 0; j < DG_NQA; ++j) rowacc += Vf[(b1 * DG_NQA + i) * nq + b2 * DG_NQA + j] * A2[j * 8 + c2];
-          acc += A1[i * 8 + c1] * rowacc;
-        }
-        Vnext[tt] = acc;
-      }
-    }
-    c.sync();
-    const int nB1 = F * nu * nq, nB2 = nu * M * 2;
-    for (int t = c.tid(); t < nB1 + nB2; t += c.nt()) {
-      if (t < nB1) {
-        // w = tv A_k + (G.p)[(ar,cr), ar-block]
-        const int f = t / (nu * nq), rem = t - f * nu * nq, rr = rem / nq, q = rem - rr * nq, b = q / DG_NQA, j = q - b * DG_NQA;
-        const int ar = rr >> 1, cr = rr & 1;
-        const double* DG_RESTRICT ABb = E.AB + (k * M + b) * 48;
-        const double* DG_RESTRICT tv = TV + (f * nu + rr) * nq + b * DG_NQA;
-        double acc = b == ar ? hc_ux(E.Hc + ((f * N + k) * M + ar) * 15, cr, j) : 0.0;
-#pragma unroll
-        for (int i = 0; i < DG_NQA; ++i) acc += tv[i] * ABb[i * 8 + j];
-        E.Wrow[(f * nq + q) * n + k * nu + rr] = acc;
-      } else {
-        // same-stage block A1 = luu + B'VB + F.p  of the functions M and a_r
-        const int e = t - nB1, rr = e / (M * 2), rem = e - rr * M * 2, b = rem >> 1, cc = rem & 1;
-        const int ar = rr >> 1, cr = rr & 1;
-        const double* DG_RESTRICT ABb = E.AB + (k * M + b) * 48;
-        double vM = 0.0, vA = 0.0;
-        const double* DG_RESTRICT tvM = TV + (M * nu + rr) * nq + b * DG_NQA;
-        const double* DG_RESTRICT tvA = TV + (ar * nu + rr) * nq + b * DG_NQA;
-#pragma unroll
-        for (int i = 0; i < DG_NQA; ++i) { vM += tvM[i] * ABb[i * 8 + 6 + cc]; vA += tvA[i] * ABb[i * 8 + 6 + cc]; }
-        if (b == ar) {
-          vM += hc_uu(E.Hc + ((M * N + k) * M + ar) * 15, cr, cc);
-          vA += hc_uu(E.Hc + ((ar * N + k) * M + ar) * 15, cr, cc);
-          if (cc == cr) vA += G.w_u[cc] + G.w_du[cc] + (k + 1 < N ? G.w_du[cc] : 0.0);
-        }
-        Qm[uidx(D, ar, k, cr) * n + uidx(D, b, k, cc)] = vA + vM;
-      }
-    }
-    c.sync();
-    double* tmp = Vcur; Vcur = Vnext; Vnext = tmp;
-  }
-}
+#include "game_kkt.cuh"
 
 // f_J at the solution (DGSQP.py:476-498, 889-893): thread per agent
 template <bool SM>
