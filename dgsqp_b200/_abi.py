@@ -67,8 +67,15 @@ class ParamsV2Struct(C.Structure):
                 ("iter_log", C.c_int32)]
 
 
+class Pcg64Struct(C.Structure):
+    """dgsqp_pcg64 (include/dgsqp_b200.h): the state of numpy.random.PCG64."""
+    _fields_ = [("state_hi", C.c_uint64), ("state_lo", C.c_uint64), ("inc_hi", C.c_uint64), ("inc_lo", C.c_uint64)]
+
+
+SAMPLE_HEAD_TO_HEAD, SAMPLE_AGENTS = 0, 1
+
 EXPORTS = ["dgsqp_create", "dgsqp_create_v2", "dgsqp_create_merge", "dgsqp_create_merge_v2", "dgsqp_destroy", "dgsqp_dims", "dgsqp_solve_batch", "dgsqp_solve_batch_up", "dgsqp_solve_batch_async",
-           "dgsqp_batch_stats", "dgsqp_last_stats", "dgsqp_pid_rollout", "dgsqp_last_diag", "dgsqp_iter_log_capacity", "dgsqp_last_iter_data", "dgsqp_phase_count", "dgsqp_last_phase_cycles", "dgsqp_measure_fp64_peak", "dgsqp_kernel_launches", "dgsqp_configure", "dgsqp_memory_plan", "dgsqp_set_smem_limit", "dgsqp_last_error", "dgsqp_version"]
+           "dgsqp_batch_stats", "dgsqp_last_stats", "dgsqp_pid_rollout", "dgsqp_sample_racing", "dgsqp_sample_merge", "dgsqp_last_diag", "dgsqp_iter_log_capacity", "dgsqp_last_iter_data", "dgsqp_phase_count", "dgsqp_last_phase_cycles", "dgsqp_measure_fp64_peak", "dgsqp_kernel_launches", "dgsqp_configure", "dgsqp_memory_plan", "dgsqp_set_smem_limit", "dgsqp_last_error", "dgsqp_version"]
 
 LIB_PATH = pathlib.Path(__file__).resolve().parent / "libdgsqp_b200.so"
 _lib = None
@@ -111,6 +118,12 @@ def load():
     lib.dgsqp_solve_batch_async.restype = C.c_int
     lib.dgsqp_pid_rollout.argtypes = [C.POINTER(RacingGameStruct), vp, C.c_int, C.c_int32, vp, vp, vp, vp, vp, vp, C.c_int32, vp]
     lib.dgsqp_pid_rollout.restype = C.c_int
+    lib.dgsqp_sample_racing.argtypes = [C.POINTER(RacingGameStruct), vp, C.c_int32, C.POINTER(Pcg64Struct), C.c_int, C.c_int32,
+                                        C.c_int64, vp, vp, vp, C.POINTER(C.c_int32), C.POINTER(C.c_int64), vp]
+    lib.dgsqp_sample_racing.restype = C.c_int
+    lib.dgsqp_sample_merge.argtypes = [C.POINTER(MergeGameStruct), C.POINTER(Pcg64Struct), C.c_int, C.c_int32, C.c_int64, vp, vp,
+                                       C.POINTER(C.c_int32), C.POINTER(C.c_int64), vp]
+    lib.dgsqp_sample_merge.restype = C.c_int
     lib.dgsqp_batch_stats.argtypes = [C.c_int, C.c_int32, vp, vp, vp, vp, vp, vp]
     lib.dgsqp_batch_stats.restype = C.c_int
     lib.dgsqp_last_stats.argtypes = [vp, vp]

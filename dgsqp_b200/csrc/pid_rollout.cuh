@@ -97,32 +97,51 @@ DG_HD double ro_pid(RoPid& c, double x, double dt) {
   return u;
 }
 
-// one agent: q0[6], xy[(N+1)*2], u_ws[N*2]
-DG_HD void ro_agent(const RolloutParams& P, double s0, double xt0, double v0, double* q0, double* xy, double* u_ws) {
-  RoPid steer = {1.0, 0.005, 0.0, P.u_ub[1], P.u_lb[1], P.rate_ub[1], P.rate_lb[1], 0.0, 0.0};
-  RoPid speed = {1.0, 0.0, v0, P.u_ub[0], P.u_lb[0], P.rate_ub[0], P.rate_lb[0], 0.0, 0.0};
-  double q[6];
-  ro_local_to_global(P, s0, xt0, q[0], q[1]);
-  q[2] = v0; q[3] = 0.0; q[4] = s0; q[5] = xt0;
-  for (int i = 0; i < 6; ++i) q0[i] = q[i];
-  xy[0] = q[0]; xy[1] = q[1];
+// one agent in flight: state, lane and speed references, and the memory of the two controllers ([0] speed, [1] steer);
+// the controller constants are re-read from P at every stage so that they need not stay in registers
+struct RoAgent { double q[6]; double xt0, v0, ei[2], u_prev[2]; };
+
+DG_HD void ro_start(const RolloutParams& P, double s0, double xt0, double v0, RoAgent& a) {
+  ro_local_to_global(P, s0, xt0, a.q[0], a.q[1]);
+  a.q[2] = v0; a.q[3] = 0.0; a.q[4] = s0; a.q[5] = xt0;
+  a.xt0 = xt0; a.v0 = v0;
+  a.ei[0] = a.ei[1] = a.u_prev[0] = a.u_prev[1] = 0.0;
+}
+
+// one stage: PID inputs (ua, us), RK4 with 4 sub-steps, then the global position from (s, e_y)
+DG_HD void ro_step(const RolloutParams& P, RoAgent& a, double& ua, double& us) {
+  double* q = a.q;
+  RoPid speed = {1.0, 0.0, a.v0, P.u_ub[0], P.u_lb[0], P.rate_ub[0], P.rate_lb[0], a.ei[0], a.u_prev[0]};
+  RoPid steer = {1.0, 0.005, 0.0, P.u_ub[1], P.u_lb[1], P.rate_ub[1], P.rate_lb[1], a.ei[1], a.u_prev[1]};
+  ua = ro_pid(speed, q[2], P.dt);
+  us = ro_pid(steer, 5.0 * (q[5] - a.xt0) + q[3], P.dt);
+  a.ei[0] = speed.ei; a.u_prev[0] = speed.u_prev;
+  a.ei[1] = steer.ei; a.u_prev[1] = steer.u_prev;
   const double h = P.dt / 4;
+  for (int sub = 0; sub < 4; ++sub) {
+    double k1[6], k2[6], k3[6], k4[6], t[6];
+    ro_fc(P, q, ua, us, k1);
+    for (int i = 0; i < 6; ++i) t[i] = q[i] + 0.5 * h * k1[i];
+    ro_fc(P, t, ua, us, k2);
+    for (int i = 0; i < 6; ++i) t[i] = q[i] + 0.5 * h * k2[i];
+    ro_fc(P, t, ua, us, k3);
+    for (int i = 0; i < 6; ++i) t[i] = q[i] + h * k3[i];
+    ro_fc(P, t, ua, us, k4);
+    for (int i = 0; i < 6; ++i) q[i] = q[i] + h / 6.0 * (k1[i] + 2 * k2[i] + 2 * k3[i] + k4[i]);
+  }
+  ro_local_to_global(P, q[4], q[5], q[0], q[1]);
+}
+
+// one agent: q0[6], xy[(N+1)*2] (may be NULL), u_ws[N*2]
+DG_HD void ro_agent(const RolloutParams& P, double s0, double xt0, double v0, double* q0, double* xy, double* u_ws) {
+  RoAgent a;
+  ro_start(P, s0, xt0, v0, a);
+  for (int i = 0; i < 6; ++i) q0[i] = a.q[i];
+  if (xy) { xy[0] = a.q[0]; xy[1] = a.q[1]; }
   for (int k = 0; k < P.N; ++k) {
-    const double ua = ro_pid(speed, q[2], P.dt);
-    const double us = ro_pid(steer, 5.0 * (q[5] - xt0) + q[3], P.dt);
-    for (int sub = 0; sub < 4; ++sub) {
-      double k1[6], k2[6], k3[6], k4[6], t[6];
-      ro_fc(P, q, ua, us, k1);
-      for (int i = 0; i < 6; ++i) t[i] = q[i] + 0.5 * h * k1[i];
-      ro_fc(P, t, ua, us, k2);
-      for (int i = 0; i < 6; ++i) t[i] = q[i] + 0.5 * h * k2[i];
-      ro_fc(P, t, ua, us, k3);
-      for (int i = 0; i < 6; ++i) t[i] = q[i] + h * k3[i];
-      ro_fc(P, t, ua, us, k4);
-      for (int i = 0; i < 6; ++i) q[i] = q[i] + h / 6.0 * (k1[i] + 2 * k2[i] + 2 * k3[i] + k4[i]);
-    }
-    ro_local_to_global(P, q[4], q[5], q[0], q[1]);
-    xy[2 * (k + 1)] = q[0]; xy[2 * (k + 1) + 1] = q[1];
+    double ua, us;
+    ro_step(P, a, ua, us);
+    if (xy) { xy[2 * (k + 1)] = a.q[0]; xy[2 * (k + 1) + 1] = a.q[1]; }
     u_ws[2 * k] = ua; u_ws[2 * k + 1] = us;
   }
 }

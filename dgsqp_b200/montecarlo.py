@@ -12,6 +12,14 @@ Instance distributions and the PID warm start follow the reference drivers
 
 ``sample_merge`` follows ``scripts/DGSQP_merge_monte_carlo.py:424-495`` (seeded, ``default_rng(1)``) and consumes
 the random stream in exactly the script's order (12 draws per trial, rejected trials included).
+
+``sample_head_to_head_cuda``, ``sample_agents_cuda`` and ``sample_merge_cuda`` draw the same distributions on the GPU
+(``dgsqp_sample_racing`` / ``dgsqp_sample_merge``, csrc/mc_sampler.cuh) and return CUDA tensors that
+``DGSQP.solve_batch`` takes on its device path.  They read ``default_rng(seed)``'s stream trial-major: trial t consumes a
+fixed block of draws (head-to-head 5, M agents 3M, merge 12) and instance i is the i-th accepted trial, so the result
+does not depend on B beyond its length.  For merge that is the order of ``sample_merge``, which the device sampler
+reproduces instance for instance; the host racing samplers above draw batch-sized blocks per quantity, so for the same
+seed they return other instances of the same distribution.
 """
 import numpy as np
 
@@ -218,3 +226,63 @@ def sample_merge(game: MergeGame, B, seed=1):
         have += len(acc)
     x0 = np.ascontiguousarray(np.vstack(out)[:B])
     return x0, np.zeros((B, game.n))
+
+
+def _pcg64_state(seed):
+    from . import _abi
+    st = np.random.default_rng(seed).bit_generator.state["state"]
+    m = (1 << 64) - 1
+    return _abi.Pcg64Struct(st["state"] >> 64, st["state"] & m, st["inc"] >> 64, st["inc"] & m)
+
+
+def _sample_cuda(game, B, seed, device, stream, max_trials, return_trials, kind):
+    import ctypes as C
+    import torch
+    from . import _abi
+    lib = _abi.load()
+    dev = torch.device("cuda", device)
+    if max_trials is None:          # four agents accept about 1 trial in 2 000
+        max_trials = max(1 << 20, 20000 * B)
+    x0 = torch.empty((B, game.n_q), dtype=torch.float64, device=dev)
+    u_ws = (torch.empty if kind is not None else torch.zeros)((B, game.n), dtype=torch.float64, device=dev)
+    trial = torch.empty(B, dtype=torch.int64, device=dev) if return_trials else None
+    if stream is None:
+        stream = torch.cuda.current_stream(dev).cuda_stream
+    acc, used = C.c_int32(0), C.c_int64(0)
+    rng = _pcg64_state(seed)
+    v = lambda t: C.c_void_p(t.data_ptr()) if t is not None and t.numel() else None
+    if kind is None:
+        rc = lib.dgsqp_sample_merge(C.byref(game.to_struct()), C.byref(rng), int(device), int(B), int(max_trials), v(x0),
+                                    v(trial), C.byref(acc), C.byref(used), C.c_void_p(stream))
+    else:
+        kp = np.ascontiguousarray(game.track.key_pts, dtype=np.float64)
+        rc = lib.dgsqp_sample_racing(C.byref(game.to_struct()), kp.ctypes.data_as(C.c_void_p), kind, C.byref(rng), int(device),
+                                     int(B), int(max_trials), v(x0), v(u_ws), v(trial), C.byref(acc), C.byref(used),
+                                     C.c_void_p(stream))
+    _abi.check(rc)
+    return (x0, u_ws, trial) if return_trials else (x0, u_ws)
+
+
+def sample_head_to_head_cuda(game: RacingGame, B, seed=0, device=0, stream=None, max_trials=None, return_trials=False):
+    """B accepted 2-agent instances drawn on the GPU: float64 CUDA tensors x0 [B,12], u_ws [B,n] agent-major (and with
+    ``return_trials`` the int64 trial id of every instance).  Same distribution and warm start as
+    :func:`sample_head_to_head`, trial-major stream (module docstring).  ``stream``: a ``cudaStream_t`` as int (default:
+    torch's current stream); ``max_trials``: give up with an error after that many trials (default
+    ``max(2^20, 20 000 B)``)."""
+    from . import _abi
+    assert game.M == 2
+    return _sample_cuda(game, B, seed, device, stream, max_trials, return_trials, _abi.SAMPLE_HEAD_TO_HEAD)
+
+
+def sample_agents_cuda(game: RacingGame, B, seed=0, device=0, stream=None, max_trials=None, return_trials=False):
+    """B accepted M-agent instances drawn on the GPU, as :func:`sample_agents` (arguments as in
+    :func:`sample_head_to_head_cuda`)."""
+    from . import _abi
+    return _sample_cuda(game, B, seed, device, stream, max_trials, return_trials, _abi.SAMPLE_AGENTS)
+
+
+def sample_merge_cuda(game: MergeGame, B, seed=1, device=0, stream=None, max_trials=None, return_trials=False):
+    """The instances of ``sample_merge(game, B, seed)`` drawn on the GPU: x0 [B, 12] (bit for bit the same) and a zero
+    warm start [B, n] as CUDA tensors (arguments as in :func:`sample_head_to_head_cuda`)."""
+    assert game.M == 3
+    return _sample_cuda(game, B, seed, device, stream, max_trials, return_trials, None)

@@ -205,6 +205,29 @@ int dgsqp_solve_batch_async(dgsqp_handle* h, int32_t B, const double* x0, const 
 int dgsqp_pid_rollout(const dgsqp_racing_game* game, const double* key_pts, int device, int32_t K, const double* s0,
                       const double* xt0, const double* v0, double* q0, double* xy, double* u_ws, int32_t memspace, void* stream);
 
+/* Monte-Carlo instance generation on the device (the sampling half of the Monte-Carlo drivers,
+ * scripts/DGSQP_ALGAMES_monte_carlo_chicane.py:384-467, DGSQP_monte_carlo_agents.py:257-308, DGSQP_merge_monte_carlo.py:424-495;
+ * host statement dgsqp_b200/montecarlo.py).  The stream is numpy.random.PCG64, started from the state of
+ * np.random.default_rng(seed).bit_generator.state.  Trial t consumes draws D*t .. D*t+D-1 (head-to-head D = 5:
+ * ego_s, ego_xt, ego_v, d, tar_v; M agents D = 3M: s, x_tran, v per agent; merge D = 12 in sample_merge's order) and
+ * instance i is the i-th accepted trial, so the output does not depend on the batch size: the first B/2 instances of a
+ * B-instance call are those of a B/2-instance call.  A trial is rejected when the PID roll-outs of its agents (see
+ * dgsqp_pid_rollout) come closer than r_i + r_j at any stage k = 0..N (head-to-head: also when the target starts behind
+ * s = 0 or off the track); merge: when the zero-input RK3 roll-outs do, car 3 rolled out from the zero state.
+ *   key_pts      HOST, as in dgsqp_pid_rollout
+ *   x0 [B, n_q]  DEVICE, state2q of the agents;  u_ws [B, n] DEVICE, PID warm start, agent-major (racing only; the merge
+ *                scenario starts from a zero warm start);  trial [B] DEVICE or NULL: trial id of every instance
+ *   accepted, trials_used  HOST: instances written, trials consumed (id of the last accepted trial + 1)
+ * Stops after max_trials trials: then returns DGSQP_EINVAL and the first *accepted rows are valid.  The call returns after
+ * the work on `stream` has completed.  Racing: M = 2..4 (head-to-head: M = 2); merge: the 3-car scenario. */
+typedef struct { uint64_t state_hi, state_lo, inc_hi, inc_lo; } dgsqp_pcg64;   /* numpy.random.PCG64 state */
+enum { DGSQP_SAMPLE_HEAD_TO_HEAD = 0, DGSQP_SAMPLE_AGENTS = 1 };
+int dgsqp_sample_racing(const dgsqp_racing_game* game, const double* key_pts, int32_t kind, const dgsqp_pcg64* rng,
+                        int device, int32_t B, int64_t max_trials, double* x0, double* u_ws, int64_t* trial,
+                        int32_t* accepted, int64_t* trials_used, void* stream);
+int dgsqp_sample_merge(const dgsqp_merge_game* game, const dgsqp_pcg64* rng, int device, int32_t B, int64_t max_trials,
+                       double* x0, int64_t* trial, int32_t* accepted, int64_t* trials_used, void* stream);
+
 /* Statistics of a solved batch reduced on the device, so that a Monte-Carlo sweep that only wants the summary table of
  * scripts/process_data_curve.py:98-110 / process_data_merge.py:58-67 does not have to copy B x (n + m) doubles back.
  * status / num_iters / qp_solves / cond are DEVICE pointers as written by dgsqp_solve_batch(memspace = 1) (cond may be

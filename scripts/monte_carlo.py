@@ -6,6 +6,9 @@
     python scripts/monte_carlo.py agents --M 3 --num 1000        # scripts/DGSQP_monte_carlo_agents.py
     python scripts/monte_carlo.py merge --num 1000 [--out merge.pkl]   # scripts/DGSQP_merge_monte_carlo.py (seed 1)
 
+--sample-on-device draws the instances on the GPU (dgsqp_b200.montecarlo.sample_*_cuda: same distributions, trial-major
+stream; for merge the same instances) and keeps them there for the solve.
+
 Prints the summary table of scripts/process_data_curve.py per cell and optionally pickles the records
 (``results['dgsqp']`` of the reference's data files)."""
 import argparse
@@ -15,7 +18,7 @@ import sys
 
 sys.path.insert(0, str(pathlib.Path(__file__).resolve().parents[1]))
 import dgsqp_b200 as dg
-from dgsqp_b200.drivers import run_monte_carlo, summary_table
+from dgsqp_b200.drivers import default_sampler, run_monte_carlo, summary_table
 
 
 def main():
@@ -28,6 +31,7 @@ def main():
     ap.add_argument("--seed", type=int, default=None)
     ap.add_argument("--device", type=int, default=0)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--sample-on-device", action="store_true", help="draw the instances on the GPU")
     a = ap.parse_args()
     cells = []
     if a.game == "chicane":
@@ -46,7 +50,8 @@ def main():
     out = {}
     for title, game, params, seed in cells:
         solver = dg.DGSQP(game, params, print_method=None, device=a.device)
-        records, stats = run_monte_carlo(solver, a.num, seed=seed if a.seed is None else a.seed)
+        sampler = default_sampler(game, device=a.device) if a.sample_on_device else None
+        records, stats = run_monte_carlo(solver, a.num, sampler=sampler, seed=seed if a.seed is None else a.seed)
         summary_table(records, title)
         out[title] = dict(dgsqp=records, stats=stats)
     if a.out:
