@@ -24,6 +24,7 @@ enum { PH_LIN_FULL = 0, PH_ADJ_FULL, PH_HESS, PH_PD_TRIDIAG, PH_PD_EIG, PH_CHOL,
 
 #ifdef DG_HOSTSIM
 #define DG_RSQRT(x) (1.0 / sqrt(x))
+#define DG_FMA(a, b, c) ((a) * (b) + (c))
 #define DG_ATOMIC_MIN(p, v) do { if ((v) < *(p)) *(p) = (v); } while (0)
 #define DG_DEV static inline
 #define DG_HD static inline
@@ -61,6 +62,8 @@ struct Cta {
 };
 #else
 #define DG_RSQRT(x) rsqrt(x)
+// a * b + c as one rounding, pinned: the compiler may not choose which product of a sum it contracts
+#define DG_FMA(a, b, c) __fma_rn((a), (b), (c))
 #define DG_ATOMIC_MIN(p, v) atomicMin((p), (v))
 #define DG_DEV __device__ __forceinline__
 #define DG_HD __host__ __device__ __forceinline__

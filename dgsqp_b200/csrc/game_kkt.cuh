@@ -33,14 +33,16 @@ DG_DEVN void game_constraints(Cta& c, const GameDesc& G, const Dims& D_, const d
   }
 }
 
-// Sensitivity rows (f_Du_x restricted to x, y, DG_BOUND_STATE): thread per input column (a, j).
+// Sensitivity rows (f_Du_x restricted to x, y, DG_BOUND_STATE): thread per input column (a, j), the agents interleaved
+// (t = j * M + a) so that the column length N - kj falls with the thread index: the last threads, which share their
+// warps with the costate chains (game_costates), hold the shortest columns.
 template <bool SM>
 DG_DEVN void game_sens(Cta& c, const Dims& D_, const EvalBuf& E_) {
   // local copies: the tables live in shared memory and would otherwise be re-read after every store
   const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
   const int twoN = D.twoN;
   DG_FOR(t, D.M * twoN) {
-    int a = t / twoN, j = t - a * twoN, kj = j >> 1, cc = j & 1;
+    int j = t / D.M, a = t - j * D.M, kj = j >> 1, cc = j & 1;
     double s[DG_NQA];
     const double* AB = E.AB + (kj * D.M + a) * DG_AB_SZ;
     for (int i = 0; i < DG_NQA; ++i) s[i] = AB[i * DG_AB_LD + DG_NQA + cc];
@@ -243,31 +245,43 @@ DG_DEV double con_lxx(const Dims& D, const double* l, int k, int i1, int i2) {
   return v;
 }
 
-// Costate chains  p_k = l_x,k + A_k' p_{k+1}:  thread per (function f, agent block b).
+// Costate chains  p_k = l_x,k + A_k' p_{k+1}:  one chain per (function f, agent block b), one lane per entry of p_k.
 // f < M: cost of agent f (terminal and stage state costs); f == M: l'C.
+// The chains are packed wsz / DG_NQA to a warp into the last warps of the CTA.  game_sens runs in the same barrier
+// interval with its longest columns on the first threads: at chicane, merge and three agents (N = 25) the chain warps
+// hold no sensitivity column at 256 threads; otherwise they share their warps with the shortest columns.
 template <bool SM>
 DG_DEVN void game_costates(Cta& c, const GameDesc& G, const Dims& D_, const EvalBuf& E_, const double* l) {
   // local copies: the tables live in shared memory and would otherwise be re-read after every store
   const EvalBuf E = E_; DG_SH_EVAL(E); const Dims D = D_;
-  DG_FOR(t, (D.M + 1) * D.M) {
-    int f = t / D.M, b = t - f * D.M;
-    double p[DG_NQA];
-    double* out = E.cst + f * (D.N + 1) * D.nq;
-    for (int i = 0; i < DG_NQA; ++i) {
-      p[i] = f < D.M ? game_term_lx(G, D, E.x, f, b * DG_NQA + i) : con_lx(G, D, E.x, l, D.N, b * DG_NQA + i);
-      out[D.N * D.nq + b * DG_NQA + i] = p[i];
-    }
-    for (int k = D.N - 1; k >= 0; --k) {
+  const int nch = (D.M + 1) * D.M;
+  const int cpw = c.wsz >= DG_NQA ? c.wsz / DG_NQA : nch;       // chains per warp (host build: all on its one thread)
+  const int ng = (nch + cpw - 1) / cpw, w = c.nwarps() - 1 - c.warp();
+  const int nown = ng > w ? (ng - w + c.nwarps() - 1) / c.nwarps() : 0;   // this warp's groups: w, w + nwarps(), ..
+  const int per = cpw * DG_NQA;
+  for (int it = c.lane(); it < nown * per; it += c.wsz) {
+    const int o = it / per, e = it - o * per, t = (w + o * c.nwarps()) * cpw + e / DG_NQA, i = e % DG_NQA;
+    if (t >= nch) continue;
+    const int f = t / D.M, b = t - f * D.M;
+    E.cst[(f * (D.N + 1) + D.N) * D.nq + b * DG_NQA + i] =
+        f < D.M ? game_term_lx(G, D, E.x, f, b * DG_NQA + i) : con_lx(G, D, E.x, l, D.N, b * DG_NQA + i);
+  }
+  c.syncwarp();
+  for (int k = D.N - 1; k >= 0; --k) {
+    for (int it = c.lane(); it < nown * per; it += c.wsz) {
+      const int o = it / per, e = it - o * per, t = (w + o * c.nwarps()) * cpw + e / DG_NQA, j = e % DG_NQA;
+      if (t >= nch) continue;
+      const int f = t / D.M, b = t - f * D.M;
       const double* Ak = E.AB + (k * D.M + b) * DG_AB_SZ;
-      double pn[DG_NQA];
-      for (int j = 0; j < DG_NQA; ++j) {
-        double acc = 0.0;
-        if (k >= 1) acc = f < D.M ? game_stage_lx(G, D, E.x, f, k, b * DG_NQA + j) : con_lx(G, D, E.x, l, k, b * DG_NQA + j);
-        for (int i = 0; i < DG_NQA; ++i) acc += Ak[i * DG_AB_LD + j] * p[i];
-        pn[j] = acc;
-      }
-      for (int i = 0; i < DG_NQA; ++i) { p[i] = pn[i]; out[k * D.nq + b * DG_NQA + i] = pn[i]; }
+      double* out = E.cst + (f * (D.N + 1) + k) * D.nq + b * DG_NQA;
+      const double* p = out + D.nq;
+      double acc = 0.0;
+      if (k >= 1) acc = f < D.M ? game_stage_lx(G, D, E.x, f, k, b * DG_NQA + j) : con_lx(G, D, E.x, l, k, b * DG_NQA + j);
+      // explicit fma(A, p, acc): a game whose l_x is a bare product (merge) must not have that product fused instead
+      for (int i = 0; i < DG_NQA; ++i) acc = DG_FMA(Ak[i * DG_AB_LD + j], p[i], acc);
+      out[j] = acc;
     }
+    c.syncwarp();
   }
 }
 
