@@ -25,6 +25,9 @@ enum { PH_LIN_FULL = 0, PH_ADJ_FULL, PH_HESS, PH_PD_TRIDIAG, PH_PD_EIG, PH_CHOL,
 #ifdef DG_HOSTSIM
 #define DG_RSQRT(x) (1.0 / sqrt(x))
 #define DG_FMA(a, b, c) ((a) * (b) + (c))
+// a * b rounded on its own, also when the host build contracts products into FMAs (tests/hostsim_lib.py, fma=True)
+static inline double dg_mul_rn(double a, double b) { volatile double r = a * b; return r; }
+#define DG_MUL(a, b) dg_mul_rn((a), (b))
 #define DG_ATOMIC_MIN(p, v) do { if ((v) < *(p)) *(p) = (v); } while (0)
 #define DG_DEV static inline
 #define DG_HD static inline
@@ -64,6 +67,8 @@ struct Cta {
 #define DG_RSQRT(x) rsqrt(x)
 // a * b + c as one rounding, pinned: the compiler may not choose which product of a sum it contracts
 #define DG_FMA(a, b, c) __fma_rn((a), (b), (c))
+// a * b rounded on its own: never contracted into a neighbouring addition
+#define DG_MUL(a, b) __dmul_rn((a), (b))
 #define DG_ATOMIC_MIN(p, v) atomicMin((p), (v))
 #define DG_DEV __device__ __forceinline__
 #define DG_HD __host__ __device__ __forceinline__

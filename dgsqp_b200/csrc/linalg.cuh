@@ -150,7 +150,10 @@ DG_DEVN void sym_tridiag(Cta& c, int n, const LinBuf& B_, int kstop) {
       }
     }
     c.sync();
-    // A22 -= v w' + w v'; the next column norm (row 0 of the updated block, columns >= 2) on the fly
+    // A22 -= v w' + w v'; the next column norm (row 0 of the updated block, columns >= 2) on the fly.  Both products are
+    // rounded on their own (DG_MUL): entries (i, j) and (j, i) then add the same two numbers and A22 stays exactly symmetric.
+    // A contracted form rounds the two entries differently; the steps below take the reflector from a column but A22 v
+    // from rows, and the asymmetry cost a degenerate cluster of eigenvalues up to 1e-4 of H (tests/test_gpu_units.py).
     nrm = 0.0;
     for (int j = sp.i0; j < len; j += sp.istep) {
       const double vj = pv[j], wj = wv[j];
@@ -165,14 +168,14 @@ DG_DEVN void sym_tridiag(Cta& c, int n, const LinBuf& B_, int kstop) {
 #pragma unroll
           for (int u = 0; u < 8; ++u) {
             const int iu = i + u * sp.G;
-            const double cv = y[u] - (pv[iu] * wj + wv[iu] * vj);
+            const double cv = y[u] - (DG_MUL(pv[iu], wj) + DG_MUL(wv[iu], vj));
             col[iu * ld] = cv;
             if (iu == 0 && j >= 2) nrm += cv * cv;
           }
         }
       }
       for (; i < len; i += sp.G) {
-        const double cv = col[i * ld] - (pv[i] * wj + wv[i] * vj);
+        const double cv = col[i * ld] - (DG_MUL(pv[i], wj) + DG_MUL(wv[i], vj));
         col[i * ld] = cv;
         if (i == 0 && j >= 2) nrm += cv * cv;
       }

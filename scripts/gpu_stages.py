@@ -1,12 +1,12 @@
 """Stage-level comparison GPU vs host build: evaluate, nearestPD, QP, LSQR dual init."""
-import sys, pathlib, ctypes as C
+import sys, pathlib
 ROOT = pathlib.Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT)); sys.path.insert(0, str(ROOT / "tests"))
 import numpy as np
 import dgsqp_b200 as dg
-from dgsqp_b200.games import params_to_struct
 from dgsqp_b200.montecarlo import sample_head_to_head
 from hostsim_lib import HostSim
+from gpu_units_lib import run_stages
 
 B = int(sys.argv[1]) if len(sys.argv) > 1 else 16
 threads = int(sys.argv[2]) if len(sys.argv) > 2 else 128
@@ -15,13 +15,9 @@ x0, u = sample_head_to_head(game, B, seed=0)
 rng = np.random.default_rng(5)
 n, m = game.n, game.m
 l = np.abs(rng.normal(size=(B, m))) * 0.3 * (rng.random((B, m)) < 0.2)
-lib = C.CDLL(str(ROOT / "tests/gpu_units/libdgsqp_units.so"))
-Q, H = np.zeros((B, n, n)), np.zeros((B, n, n)); q, gtl, du = (np.zeros((B, n)) for _ in range(3))
-g, lam, l0 = (np.zeros((B, m)) for _ in range(3)); nneg, qpst, qpit, lit = (np.zeros(B, dtype=np.int32) for _ in range(4))
-p = lambda a: a.ctypes.data_as(C.c_void_p)
-gs, ps = game.to_struct(), params_to_struct(params)
-rc = lib.units_run(C.byref(gs), C.byref(ps), B, threads, p(x0), p(u), p(l), p(Q), p(q), p(gtl), p(g), p(H), p(du), p(lam), p(l0), p(nneg), p(qpst), p(qpit), p(lit))
-assert rc == 0, rc
+o = run_stages(game, params, x0, u, l, threads=threads)
+Q, q, gtl, g, H, du, lam, l0 = (o[k] for k in ("Q", "q", "gtl", "g", "H", "du", "lam", "l0"))
+nneg, qpst, qpit, lit = o["nneg"], o["qpst"], o["qpit"], o["lsqr_it"]
 hs = HostSim(game, params)
 for i in range(B):
     Qh, qh, gtlh, gh, xh = hs.evaluate(x0[i], u[i], l[i])

@@ -22,7 +22,7 @@ extern "C" int hs_pid_rollout(const dgsqp_racing_game* g, const double* key_pts,
 
 extern "C" {
 
-struct HsHandle { GameDesc G; SolverParams P; Dims D; std::vector<double> ws, sh; Workspace W; std::vector<double*> guards; };
+struct HsHandle { GameDesc G; SolverParams P; Dims D; std::vector<double> ws, sh; Workspace W; MemPlan plan; std::vector<double*> guards; };
 static const double HS_CANARY = -7.25e77;
 
 static void* hs_create_common(const dg_game_struct* g, const dgsqp_params* p, const dgsqp_v2_params* p2) {
@@ -33,6 +33,7 @@ static void* hs_create_common(const dg_game_struct* g, const dgsqp_params* p, co
   const char* lim = getenv("DG_HOSTSIM_SMEM_DOUBLES");      // tests cover both placements
   size_t budget = lim ? (size_t)atol(lim) : 28000;
   MemPlan pl = plan_memory(h->D, nullptr, nullptr, budget, tmp);
+  h->plan = pl;
   h->ws.assign(pl.gmem + 2, 0.0);
   h->sh.assign(pl.smem + 2, 0.0);
 #ifdef DG_PLAN_GUARD
@@ -65,6 +66,12 @@ int hs_guard_check(void* hp) {
 void hs_set_l0_perturb(void* hp, double v) { ((HsHandle*)hp)->P.dbg_l0_perturb = v; }
 void hs_destroy(void* hp) { delete (HsHandle*)hp; }
 void hs_dims(void* hp, int* out) { HsHandle* h = (HsHandle*)hp; out[0] = h->D.nq; out[1] = h->D.nu; out[2] = h->D.n; out[3] = h->D.m; }
+// memory plan: {hot_in_smem, mats_in_smem, matA_in_smem, sens_in_smem, eig_s set} (as tests/gpu_units/units.cu reports it)
+void hs_plan(void* hp, int* out) {
+  HsHandle* h = (HsHandle*)hp;
+  out[0] = h->plan.hot_in_smem; out[1] = h->plan.mats_in_smem; out[2] = h->plan.matA_in_smem; out[3] = h->plan.sens_in_smem;
+  out[4] = h->W.B.eig_s != nullptr;
+}
 
 // full evaluation at (u, l): returns Q[n*n], q[n], gtl[n], g[m], x
 void hs_evaluate(void* hp, const double* x0, const double* u, const double* l, double* Q, double* q, double* gtl,
@@ -93,16 +100,35 @@ int hs_nearest_pd(void* hp, const double* Qin, double* Hout) {
   for (int i = 0; i < h->D.n; ++i) memcpy(Hout + (size_t)i * h->D.n, h->W.B.matA + (size_t)i * h->D.ld, sizeof(double) * h->D.n);
   return nn;
 }
-// QP at the last evaluated point with the given H (n*n, destroyed) and q
-int hs_qp(void* hp, double* H, const double* q, double* du, double* lam, int* iters) {
-  HsHandle* h = (HsHandle*)hp; Cta c;
+// QP at the last evaluated point with the given H (n*n, destroyed) and q; warm != 0 starts from the active set of the
+// previous QP of this handle
+static int hs_qp_common(HsHandle* h, double* H, const double* q, double* du, double* lam, int* iters, int warm) {
+  Cta c;
   int na = 0;
   for (int i = 0; i < h->D.n; ++i) memcpy(h->W.B.matA + (size_t)i * h->D.ld, H + (size_t)i * h->D.n, sizeof(double) * h->D.n);
   std::vector<double> qc(q, q + h->D.n);      // q may alias workspace the solver reuses
-  int st = qp_solve_gi<false>(c, h->D, h->W.E, qc.data(), h->W.Q, h->W.B, iters, &na, 0);
+  int st = qp_solve_gi<false>(c, h->D, h->W.E, qc.data(), h->W.Q, h->W.B, iters, &na, warm);
   memcpy(du, h->W.Q.xq, sizeof(double) * h->D.n);
   memcpy(lam, h->W.Q.lam, sizeof(double) * h->D.m);
   return st;
+}
+int hs_qp(void* hp, double* H, const double* q, double* du, double* lam, int* iters) { return hs_qp_common((HsHandle*)hp, H, q, du, lam, iters, 0); }
+int hs_qp_warm(void* hp, double* H, const double* q, double* du, double* lam, int* iters) { return hs_qp_common((HsHandle*)hp, H, q, du, lam, iters, 1); }
+// qp_factor of H (n*n): returns ok; L (lower triangle, zero above), Y = L^-1 (all n x n entries as stored), xq = -H^-1 q
+int hs_factor(void* hp, const double* H, const double* q, double* L, double* Y, double* xq) {
+  HsHandle* h = (HsHandle*)hp; Cta c;
+  const int n = h->D.n, ld = h->D.ld;
+  for (int i = 0; i < n; ++i) memcpy(h->W.B.matA + (size_t)i * ld, H + (size_t)i * n, sizeof(double) * n);
+  for (size_t t = 0; t < (size_t)n * ld; ++t) h->W.B.matB[t] = 3.0;    // the factorisation must write Y's zero upper triangle
+  std::vector<double> qc(q, q + n);
+  const bool ok = qp_factor<false>(c, h->D, qc.data(), h->W.Q, h->W.B);
+  for (int i = 0; i < n; ++i)
+    for (int j = 0; j < n; ++j) {
+      L[(size_t)i * n + j] = j <= i ? h->W.B.matA[(size_t)i * ld + j] : 0.0;
+      Y[(size_t)i * n + j] = h->W.B.matB[(size_t)i * ld + j];
+    }
+  memcpy(xq, h->W.Q.xq, sizeof(double) * n);
+  return ok;
 }
 int hs_lsqr(void* hp, const double* x0, const double* u, double* l_out) {
   HsHandle* h = (HsHandle*)hp; Cta c;

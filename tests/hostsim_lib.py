@@ -14,9 +14,9 @@ HERE = pathlib.Path(__file__).resolve().parent / "hostsim"
 _libs = {}
 
 
-def build(asan=False, merge=False, guard=False):
+def build(asan=False, merge=False, guard=False, fma=False):
     out = HERE / ("libhostsim" + ("_merge" if merge else "") + ("_asan" if asan else "") + ("_guard" if guard else "")
-                  + ".so")
+                  + ("_fma" if fma else "") + ".so")
     srcs = [HERE / "hostsim.cpp"] + sorted((HERE.parents[1] / "dgsqp_b200" / "csrc").glob("*.cuh")) \
         + sorted((HERE.parents[1] / "dgsqp_b200" / "csrc").glob("*.h"))
     if out.exists() and all(out.stat().st_mtime >= s.stat().st_mtime for s in srcs):
@@ -26,28 +26,32 @@ def build(asan=False, merge=False, guard=False):
         flags = flags + ["-DDG_GAME_MERGE=1"]
     if guard:
         flags = flags + ["-DDG_PLAN_GUARD=16"]      # canary gaps behind every buffer of the memory plan (hs_guard_check)
+    if fma:
+        flags = flags + ["-mfma", "-ffp-contract=fast"]   # products contracted into FMAs wherever the compiler likes, as nvcc does
     subprocess.check_call(["g++", *flags, "-shared", "-fPIC", "-std=c++17", "-o", str(out), str(HERE / "hostsim.cpp")])
     return out
 
 
-def load(asan=False, merge=False, guard=False):
-    if (asan, merge, guard) in _libs:
-        return _libs[(asan, merge, guard)]
-    lib = C.CDLL(str(build(asan, merge, guard)))
+def load(asan=False, merge=False, guard=False, fma=False):
+    if (asan, merge, guard, fma) in _libs:
+        return _libs[(asan, merge, guard, fma)]
+    lib = C.CDLL(str(build(asan, merge, guard, fma)))
     gs = MergeGameStruct if merge else RacingGameStruct
     lib.hs_create.restype = C.c_void_p
     lib.hs_create.argtypes = [C.POINTER(gs), C.POINTER(ParamsStruct)]
     lib.hs_create_v2.restype = C.c_void_p
     lib.hs_create_v2.argtypes = [C.POINTER(gs), C.POINTER(ParamsV2Struct)]
     for name in ["hs_destroy", "hs_dims", "hs_evaluate", "hs_G_dense", "hs_G_times", "hs_GT_times", "hs_nearest_pd",
-                 "hs_qp", "hs_lsqr", "hs_solve"]:
+                 "hs_qp", "hs_qp_warm", "hs_factor", "hs_plan", "hs_lsqr", "hs_solve"]:
         getattr(lib, name).argtypes = None
     lib.hs_nearest_pd.restype = C.c_int
     lib.hs_qp.restype = C.c_int
+    lib.hs_qp_warm.restype = C.c_int
+    lib.hs_factor.restype = C.c_int
     lib.hs_lsqr.restype = C.c_int
     lib.hs_guard_check.restype = C.c_int
     lib.hs_guard_check.argtypes = [C.c_void_p]
-    _libs[(asan, merge, guard)] = lib
+    _libs[(asan, merge, guard, fma)] = lib
     return lib
 
 
@@ -56,8 +60,8 @@ def _p(a):
 
 
 class HostSim:
-    def __init__(self, game, params, asan=False, guard=False, qp_warm=True, mu_vio_thresh=1e-10):
-        self.lib = load(asan, merge=isinstance(game, MergeGame), guard=guard)
+    def __init__(self, game, params, asan=False, guard=False, qp_warm=True, mu_vio_thresh=1e-10, fma=False):
+        self.lib = load(asan, merge=isinstance(game, MergeGame), guard=guard, fma=fma)
         self.game = game
         gs = game.to_struct()
         if isinstance(params, DGSQPV2Params):
@@ -118,6 +122,29 @@ class HostSim:
         it = C.c_int(0)
         st = self.lib.hs_qp(self.h, _p(H), _p(q), _p(du), _p(lam), C.byref(it))
         return st, du, lam, it.value
+
+    def qp_warm(self, H, q):
+        """QP at (H, q) started from the active set of the previous QP of this handle (gi_warm_start)."""
+        H = np.ascontiguousarray(H, dtype=np.float64).copy()
+        q = np.ascontiguousarray(q, dtype=np.float64)
+        du, lam = np.zeros(self.n), np.zeros(self.m)
+        it = C.c_int(0)
+        st = self.lib.hs_qp_warm(self.h, _p(H), _p(q), _p(du), _p(lam), C.byref(it))
+        return st, du, lam, it.value
+
+    def factor(self, H, q):
+        """qp_factor: (ok, L, Y = L^-1 as stored, xq = -H^-1 q)."""
+        H = np.ascontiguousarray(H, dtype=np.float64)
+        q = np.ascontiguousarray(q, dtype=np.float64)
+        L, Y, xq = np.zeros((self.n, self.n)), np.zeros((self.n, self.n)), np.zeros(self.n)
+        ok = self.lib.hs_factor(self.h, _p(H), _p(q), _p(L), _p(Y), _p(xq))
+        return bool(ok), L, Y, xq
+
+    def plan(self):
+        """Memory plan: (hot_in_smem, mats_in_smem, matA_in_smem, sens_in_smem, eig_s set)."""
+        out = np.zeros(5, dtype=np.int32)
+        self.lib.hs_plan(self.h, _p(out))
+        return tuple(int(v) for v in out)
 
     def lsqr(self, x0, u):
         l = np.zeros(self.m)

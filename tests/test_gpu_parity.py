@@ -20,25 +20,50 @@ def _rel(a, b):
 
 
 # ------------------------------------------------------------------ stage level (K1..K3, K0)
-@pytest.mark.parametrize("threads", [64, 128, 256])
-def test_stages_vs_oracle(threads):
+def _stage_game(name):
+    """(game, params, oracle game, sampler) of the stage-level checks."""
+    from dgsqp_b200.montecarlo import sample_merge
+    from oracle.merge_game import MergeGame
+    from oracle.racing_game import RacingGame
+    from oracle.track import chicane_track, curve_track
+    if name == "chicane":
+        return dg.chicane_game(), dg.chicane_params(), RacingGame(chicane_track(), M=2, N=25), \
+            lambda g, B: sample_head_to_head(g, B, seed=11)
+    if name == "merge":
+        return dg.merge_game(), dg.merge_params(), MergeGame(N=20), lambda g, B: sample_merge(g, B, seed=1)
+    M = int(name[-1])
+    return dg.agents_game(M, 90.0, 25), dg.agents_params(25), \
+        RacingGame(curve_track(curve_angle=np.pi / 2), M=M, N=25, obs_r=0.4), lambda g, B: sample_agents(g, B, seed=0)
+
+
+# shared-memory budgets (doubles): the default; matA in shared memory and matB in L2 (chicane and merge only: the
+# matrices of the agent games do not fit); everything in the global workspace
+_STAGE_BUDGETS = {"default": {}, "split": {"chicane": 23000, "merge": 27000}, "global": {}}
+
+
+def _stages_vs_oracle(name, threads, budget="default"):
     """Rollout+derivatives, KKT assembly, eigen-projection, QP and LSQR of the CUDA path, each against the
-    oracle on the same inputs (chicane, N = 25)."""
+    oracle on the same inputs."""
     from gpu_units_lib import run_stages
     from oracle.dgsqp_v1 import OracleDGSQP, nearest_pd
     from oracle.qp import solve_qp_gi, kkt_residuals
-    from oracle.racing_game import RacingGame
-    from oracle.track import chicane_track
-    game, params = dg.chicane_game(), dg.chicane_params()
-    og = RacingGame(chicane_track(), M=2, N=25)
+    game, params, og, sampler = _stage_game(name)
     B = 6
-    x0, u = sample_head_to_head(game, B, seed=11)
+    x0, u = sampler(game, B)
     rng = np.random.default_rng(5)
+    if name == "merge":                                 # the merge warm start is u = 0
+        u = rng.normal(size=u.shape) * 0.15
     l = np.abs(rng.normal(size=(B, game.m))) * 0.3 * (rng.random((B, game.m)) < 0.2)
-    out = run_stages(game, params, x0, u, l, threads=threads)
-    sol = OracleDGSQP(og)
+    lim = {"default": None, "global": 0}.get(budget, _STAGE_BUDGETS[budget].get(name))
+    out = run_stages(game, params, x0, u, l, threads=threads, smem_limit_doubles=lim)
+    plan = out["plan"]
+    if budget == "split":
+        assert plan["matA_in_smem"] and not plan["mats_in_smem"]
+    if budget == "global":
+        assert not plan["matA_in_smem"] and not plan["hot_in_smem"]
+    sol = OracleDGSQP(og, reg=params.reg)
     for i in range(B):
-        Q, q, G, g, _ = og.evaluate(u[i], l[i], x0[i], np.zeros(4), True)
+        Q, q, G, g, _ = og.evaluate(u[i], l[i], x0[i], np.zeros(og.n_u), True)
         assert _rel(out["Q"][i], Q) < 1e-12 and _rel(out["q"][i], q) < 1e-12
         assert _rel(out["gtl"][i], G.T @ l[i]) < 1e-12 and _rel(out["g"][i], g) < 1e-13
         H = nearest_pd(Q) + params.reg * np.eye(game.n)
@@ -49,10 +74,27 @@ def test_stages_vs_oracle(threads):
         assert _rel(out["du"][i], du) < 1e-8 and _rel(out["lam"][i], lam) < 1e-7
         r = kkt_residuals(H, q, G, g, out["du"][i], out["lam"][i])
         assert r["stat"] < 1e-8 and r["feas"] < 1e-9 and r["dual"] == 0.0 and r["comp"] < 1e-8
-        q0, G0, _, _ = og.evaluate(u[i], np.zeros(game.m), x0[i], np.zeros(4), False)
+        q0, G0, _, _ = og.evaluate(u[i], np.zeros(game.m), x0[i], np.zeros(og.n_u), False)
         l0 = sol.dual_init(q0, G0)
         assert int(out["lsqr_it"][i]) == sol.lsqr_iters
         assert np.abs(out["l0"][i] - l0).max() < 1e-9 * max(1.0, np.abs(l0).max())
+
+
+@pytest.mark.parametrize("threads", [64, 128, 256])
+def test_stages_vs_oracle(threads):
+    """Every stage of the CUDA path against the oracle on the same inputs (chicane, N = 25)."""
+    _stages_vs_oracle("chicane", threads)
+
+
+@pytest.mark.parametrize("name,threads,budget", [
+    ("chicane", 256, "split"), ("chicane", 128, "global"), ("chicane", 96, "default"),
+    ("merge", 256, "default"), ("merge", 64, "split"), ("merge", 128, "global"),
+    ("agents3", 256, "default"), ("agents3", 96, "global"),
+    ("agents4", 256, "default"), ("agents4", 64, "default"), ("agents4", 128, "global")])
+def test_stages_vs_oracle_games_and_placements(name, threads, budget):
+    """The same stage checks on the merge game and the three- and four-agent races, in the three memory placements
+    (agents4 at 64 threads: more costate chain groups than warps)."""
+    _stages_vs_oracle(name, threads, budget)
 
 
 # ------------------------------------------------------------------ full solves vs golden (oracle) results
