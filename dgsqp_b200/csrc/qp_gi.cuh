@@ -367,9 +367,10 @@ DG_DEVN int gi_warm_start(Cta& c, const Dims& D_, const EvalBuf& E_, const doubl
     c.lapf(PH_WS_QR);
     const int knext = kk + pa + dep;
     if (pa > 0) {
-      // block reflector on the columns of Y, the remaining source columns and c: thread per target column, the three
-      // kinds of target on different warps
-      const int p0 = iq, nrem = nprev - knext;
+      // block reflector on the columns of Y, the source columns behind the panel and c: thread per target column, the
+      // three kinds of target on different warps.  The panel's own columns after a dependent one (knext .. kk + pw)
+      // already carry the panel's reflectors (the in-panel updates above); a second application would undo them.
+      const int kend = nprev - kk < PW ? nprev : kk + PW, p0 = iq, nrem = nprev - kend;      // kk + pw
       const int sD = (n + c.wsz - 1) / c.wsz * c.wsz, sC = sD + (nrem + c.wsz - 1) / c.wsz * c.wsz;
       const double* DG_RESTRICT V = Rm + kk;
       const bool pad8 = kk + PW <= ld && p0 + PW <= n;
@@ -377,12 +378,12 @@ DG_DEVN int gi_warm_start(Cta& c, const Dims& D_, const EvalBuf& E_, const doubl
       for (int slot = c.tid(); slot <= sC; slot += c.nt()) {
         if (pad8) {
           if (slot < n) ws_apply_panel<true, RBY>(Y + slot, ld, V, ld, p0, pa, n, v0s + p0, scs + p0, gram);
-          else if (slot >= sD && slot - sD < nrem) ws_apply_panel<true, 2>(Rm + knext + (slot - sD), ld, V, ld, p0, pa, n, v0s + p0, scs + p0, gram);
+          else if (slot >= sD && slot - sD < nrem) ws_apply_panel<true, 2>(Rm + kend + (slot - sD), ld, V, ld, p0, pa, n, v0s + p0, scs + p0, gram);
           else if (slot == sC) ws_apply_panel<true, 2>(cv, 1, V, ld, p0, pa, n, v0s + p0, scs + p0, gram);
         } else {
           double* DG_RESTRICT tp = nullptr; int st = ld;
           if (slot < n) tp = Y + slot;
-          else if (slot >= sD && slot - sD < nrem) tp = Rm + knext + (slot - sD);
+          else if (slot >= sD && slot - sD < nrem) tp = Rm + kend + (slot - sD);
           else if (slot == sC) { tp = cv; st = 1; }
           if (tp) ws_apply_panel<false, 2>(tp, st, V, ld, p0, pa, n, v0s + p0, scs + p0, gram);
         }

@@ -37,7 +37,7 @@ def solve_qp_gi(H, q, G, g, max_iter=None, feas_tol=FEAS_TOL, stats=None, polish
     lam_act = np.zeros(0)
     iq = 0
     it = 0
-    n_add = n_drop = 0
+    n_add = n_drop = n_drop_dep = 0
     while True:
         s = -g - G @ x
         if iq:
@@ -115,6 +115,7 @@ def solve_qp_gi(H, q, G, g, max_iter=None, feas_tol=FEAS_TOL, stats=None, polish
             lam_act = np.delete(lam_act, ldrop)
             iq -= 1
             n_drop += 1
+            n_drop_dep += not np.isfinite(t2)           # p dependent on the active set: a pure dual step
     # Polish.  The iteration starts at the unconstrained minimiser x0 = -H^-1 q and moves by x += t z; for an
     # ill-conditioned H (reg = 0 games: eigenvalues at the 1e-10 floor) x0 is ~1e10 |q| along the near-null directions and
     # the steps cancel it, leaving errors of 1e-5..1e-3 in x and 1e-2 in lam.  The KKT point of the final active set W is
@@ -134,7 +135,7 @@ def solve_qp_gi(H, q, G, g, max_iter=None, feas_tol=FEAS_TOL, stats=None, polish
     if iq:
         lam[act] = lam_act
     if stats is not None:
-        stats.update(iters=it, n_add=n_add, n_drop=n_drop, n_active=iq)
+        stats.update(iters=it, n_add=n_add, n_drop=n_drop, n_drop_dep=n_drop_dep, n_active=iq)
     return x, lam
 
 

@@ -1,7 +1,8 @@
 // Stage-level test kernel: runs single stages of the solver -- evaluate -> nearestPD -> QP and the LSQR dual
 // initialisation, nearestPD of an arbitrary matrix, the QP factorisation, a cold and a warm QP with an arbitrary
-// Hessian, the matrix-free G products -- for a batch of instances (one CTA each) and returns every intermediate
-// together with the memory plan it ran with.  TEST ONLY (tests/test_gpu_units.py, tests/test_gpu_parity.py).
+// Hessian (and optionally arbitrary constraint offsets and warm-start list), the warm start alone, the matrix-free G
+// products -- for a batch of instances (one CTA each) and returns every intermediate together with the memory plan it
+// ran with.  TEST ONLY (tests/test_gpu_units.py, tests/test_gpu_qp.py, tests/test_gpu_parity.py).
 // Compiled once per game: -DDG_GAME_MERGE selects the merge game (csrc/game.cuh).
 #include <cuda_runtime.h>
 #include <cstdio>
@@ -9,15 +10,17 @@
 #include "../../dgsqp_b200/csrc/sqp_v1.cuh"
 #include "../../dgsqp_b200/csrc/host_setup.h"
 
-enum { U_STAGES = 0, U_NEAREST_PD = 1, U_FACTOR = 2, U_QP = 3, U_G = 4 };
+enum { U_STAGES = 0, U_NEAREST_PD = 1, U_FACTOR = 2, U_QP = 3, U_G = 4, U_WARM = 5 };
 
 struct UnitArgs {
   int B, mode, nrows;
   const double *x0, *u, *l;              // evaluation point (U_STAGES, U_QP, U_G)
   const double *Hin, *qin, *q2in;        // nearestPD input (U_NEAREST_PD); QP Hessian and gradients (U_FACTOR, U_QP)
   const double *v, *w; const int* rows;  // U_G: G v, G' w, rows / columns of G
-  double *Q, *q, *gtl, *g, *H, *du, *lam, *l0, *du2, *lam2, *L, *Y, *Gv, *GTw, *Grow, *Gcol;
-  int *nneg, *qpst, *qpit, *lsqr_it, *qpst2, *qpit2, *ok, *eig_s;
+  const double* gin;                     // U_QP, U_WARM: constraint offsets [B, m] in place of the evaluated g (or null)
+  const int *prev, *kprev; int kmax;     // U_QP, U_WARM: warm-start list prev[B, kmax], kprev[b] ids of it (or null)
+  double *Q, *q, *gtl, *g, *H, *du, *lam, *l0, *du2, *lam2, *L, *Y, *Gv, *GTw, *Grow, *Gcol, *lam_act;
+  int *nneg, *qpst, *qpit, *lsqr_it, *qpst2, *qpit2, *qpna, *qpna2, *ok, *eig_s, *act, *iq;
   double* ws; size_t ws_stride; size_t smem_doubles;
 };
 
@@ -42,7 +45,7 @@ __global__ void __launch_bounds__(256, 1) units_kernel(const GameDesc* Gp, const
     c.sync();
     const double* u = A.u ? A.u + (size_t)inst * n : nullptr;
     const double* l = A.l ? A.l + (size_t)inst * m : nullptr;
-    if (A.mode == U_STAGES || A.mode == U_QP || A.mode == U_G) {
+    if (A.mode == U_STAGES || A.mode == U_QP || A.mode == U_G || A.mode == U_WARM) {
       if (threadIdx.x == 0) X.x0 = A.x0 + (size_t)inst * D.nq;
       DG_FOR(j, D.nu) X.W.S.up[j] = 0.0;
       c.sync();
@@ -51,6 +54,11 @@ __global__ void __launch_bounds__(256, 1) units_kernel(const GameDesc* Gp, const
       DG_FOR(t, n * n) A.Q[(size_t)inst * n * n + t] = X.W.E.Q[t];
       DG_FOR(t, n) { A.q[(size_t)inst * n + t] = X.W.E.q[t]; A.gtl[(size_t)inst * n + t] = X.W.E.gtl[t]; }
       DG_FOR(t, m) A.g[(size_t)inst * m + t] = X.W.E.g[t];
+      c.sync();
+      if (A.gin) { DG_FOR(t, m) X.W.E.g[t] = A.gin[(size_t)inst * m + t]; }
+      const int kp = A.prev ? A.kprev[inst] : 0;
+      DG_FOR(t, kp) X.W.Q.act[t] = A.prev[(size_t)inst * A.kmax + t];
+      if (c.tid() == 0) X.W.Q.act[n] = kp;
       c.sync();
     }
     if (A.mode == U_STAGES) {
@@ -92,21 +100,41 @@ __global__ void __launch_bounds__(256, 1) units_kernel(const GameDesc* Gp, const
       DG_FOR(t, n) A.du[(size_t)inst * n + t] = X.W.Q.xq[t];
       if (c.tid() == 0) A.ok[inst] = ok;
     } else if (A.mode == U_QP) {
-      // cold QP at (H, q) on the evaluated constraints; then, with q2, a warm QP from the cold QP's active set
+      // QP at (H, q) on the evaluated constraints (or on gin), cold or from the list prev; then, with q2, a warm QP
+      // from the first QP's active set
       for (int pass = 0; pass < (A.q2in ? 2 : 1); ++pass) {
         const double* qi = (pass == 0 ? A.qin : A.q2in) + (size_t)inst * n;
         DG_FOR(t, n * n) matA[(t / n) * ld + (t % n)] = A.Hin[(size_t)inst * n * n + t];
         DG_FOR(t, n) X.W.E.q[t] = qi[t];
-        if (pass == 0 && c.tid() == 0) X.W.Q.act[n] = 0;
         c.sync();
         int it = 0, na = 0;
-        const int st = qp_solve_gi<SM>(c, D, X.W.E, X.W.E.q, X.W.Q, X.W.B, &it, &na, pass);
+        const int st = qp_solve_gi<SM>(c, D, X.W.E, X.W.E.q, X.W.Q, X.W.B, &it, &na, pass > 0 || A.prev);
         c.sync();
         DG_FOR(t, n) (pass == 0 ? A.du : A.du2)[(size_t)inst * n + t] = X.W.Q.xq[t];
         DG_FOR(t, m) (pass == 0 ? A.lam : A.lam2)[(size_t)inst * m + t] = X.W.Q.lam[t];
-        if (c.tid() == 0) { (pass == 0 ? A.qpst : A.qpst2)[inst] = st; (pass == 0 ? A.qpit : A.qpit2)[inst] = it; }
+        if (c.tid() == 0) {
+          (pass == 0 ? A.qpst : A.qpst2)[inst] = st; (pass == 0 ? A.qpit : A.qpit2)[inst] = it;
+          (pass == 0 ? A.qpna : A.qpna2)[inst] = na;
+        }
         c.sync();
       }
+    } else if (A.mode == U_WARM) {
+      // qp_factor and gi_warm_start from prev only: the S-pair (act[0..iq), xq, lam_act[0..iq)) the main loop starts from
+      DG_FOR(t, n * n) matA[(t / n) * ld + (t % n)] = A.Hin[(size_t)inst * n * n + t];
+      DG_FOR(t, n) X.W.E.q[t] = A.qin[(size_t)inst * n + t];
+      c.sync();
+      int iq = -1;
+      if (qp_factor<SM>(c, D, X.W.E.q, X.W.Q, X.W.B)) {
+        const int kp = X.W.Q.act[n];
+        iq = kp > 0 ? gi_warm_start<SM>(c, D, X.W.E, X.W.E.q, X.W.Q, X.W.B, kp) : 0;
+      }
+      c.sync();
+      DG_FOR(t, n) A.du[(size_t)inst * n + t] = X.W.Q.xq[t];
+      DG_FOR(t, n) {
+        A.act[(size_t)inst * n + t] = t < iq ? X.W.Q.act[t] : -1;
+        A.lam_act[(size_t)inst * n + t] = t < iq ? X.W.Q.lam_act[t] : 0.0;
+      }
+      if (c.tid() == 0) A.iq[inst] = iq;
     } else if (A.mode == U_G) {
       // the operands go where the solver keeps them (SQP iterate vectors, QP scratch, matA)
       DG_FOR(t, n) X.W.S.du[t] = A.v[(size_t)inst * n + t];
@@ -246,19 +274,57 @@ int units_factor(const dg_game_struct* game, const dgsqp_params* params, int B, 
   return units_launch(game, params, threads, smem_limit_doubles, A, da, plan);
 }
 
-// evaluation at (x0, u, l) (constraints of the QP), a cold QP at (H, q) and, if q2 is given, a warm QP at (H, q2)
-// from the cold QP's active set
+// the optional constraint offsets gin[B, m] and warm-start lists prev[B, kmax] (kprev[b] ids each) of U_QP / U_WARM
+static int units_qp_inputs(const Dims& D, int B, const double* gin, const int* prev, const int* kprev, int kmax,
+                           UnitArgs& A, DevArrays& da) {
+  if (prev) {
+    if (!kprev || kmax < 1 || kmax > D.n) return -1;
+    for (int b = 0; b < B; ++b) {
+      if (kprev[b] < 0 || kprev[b] > kmax) return -1;
+      for (int k = 0; k < kprev[b]; ++k) if (prev[(size_t)b * kmax + k] < 0 || prev[(size_t)b * kmax + k] >= D.m) return -1;
+    }
+    A.prev = da.in(prev, (size_t)B * kmax); A.kprev = da.in(kprev, B); A.kmax = kmax;
+  }
+  A.gin = da.in(gin, (size_t)B * D.m);
+  return 0;
+}
+
+// evaluation at (x0, u, l) (constraints of the QP, offsets replaced by gin if given), a QP at (H, q) -- cold, or from
+// the warm-start list prev if given -- and, if q2 is given, a warm QP at (H, q2) from the first QP's active set.
+// it / na: main-loop iterations and active rows at the end
 int units_qp(const dg_game_struct* game, const dgsqp_params* params, int B, int threads, long smem_limit_doubles,
              const double* x0, const double* u, const double* l, const double* H, const double* q, const double* q2,
-             double* Q, double* qe, double* gtl, double* g, int* st, int* it, double* du, double* lam,
-             int* st2, int* it2, double* du2, double* lam2, int* plan) {
+             const double* gin, const int* prev, const int* kprev, int kmax,
+             double* Q, double* qe, double* gtl, double* g, int* st, int* it, int* na, double* du, double* lam,
+             int* st2, int* it2, int* na2, double* du2, double* lam2, int* plan) {
   const Dims D = units_dims(game); const size_t n = D.n, m = D.m;
   DevArrays da; UnitArgs A = units_args(B, U_QP);
+  if (units_qp_inputs(D, B, gin, prev, kprev, kmax, A, da)) return -1;
   A.x0 = da.in(x0, B * D.nq); A.u = da.in(u, B * n); A.l = da.in(l, B * m);
   A.Hin = da.in(H, B * n * n); A.qin = da.in(q, B * n); A.q2in = da.in(q2, B * n);
   A.Q = da.out(Q, B * n * n); A.q = da.out(qe, B * n); A.gtl = da.out(gtl, B * n); A.g = da.out(g, B * m);
-  A.qpst = da.out(st, B); A.qpit = da.out(it, B); A.du = da.out(du, B * n); A.lam = da.out(lam, B * m);
-  if (q2) { A.qpst2 = da.out(st2, B); A.qpit2 = da.out(it2, B); A.du2 = da.out(du2, B * n); A.lam2 = da.out(lam2, B * m); }
+  A.qpst = da.out(st, B); A.qpit = da.out(it, B); A.qpna = da.out(na, B); A.du = da.out(du, B * n); A.lam = da.out(lam, B * m);
+  if (q2) {
+    A.qpst2 = da.out(st2, B); A.qpit2 = da.out(it2, B); A.qpna2 = da.out(na2, B);
+    A.du2 = da.out(du2, B * n); A.lam2 = da.out(lam2, B * m);
+  }
+  return units_launch(game, params, threads, smem_limit_doubles, A, da, plan);
+}
+
+// evaluation at (x0, u, l) (offsets replaced by gin if given), qp_factor of H and gi_warm_start from prev: iq (-1: H
+// not positive definite), act[B, n] (-1 from iq on), xq[B, n], lam_act[B, n] (0 from iq on)
+int units_warm(const dg_game_struct* game, const dgsqp_params* params, int B, int threads, long smem_limit_doubles,
+               const double* x0, const double* u, const double* l, const double* H, const double* q,
+               const double* gin, const int* prev, const int* kprev, int kmax,
+               int* iq, int* act, double* xq, double* lam_act, int* plan) {
+  const Dims D = units_dims(game); const size_t n = D.n, m = D.m;
+  DevArrays da; UnitArgs A = units_args(B, U_WARM);
+  if (!prev || units_qp_inputs(D, B, gin, prev, kprev, kmax, A, da)) return -1;
+  A.x0 = da.in(x0, B * D.nq); A.u = da.in(u, B * n); A.l = da.in(l, B * m);
+  A.Hin = da.in(H, B * n * n); A.qin = da.in(q, B * n);
+  A.iq = da.out(iq, B); A.act = da.out(act, B * n); A.du = da.out(xq, B * n); A.lam_act = da.out(lam_act, B * n);
+  // the evaluation outputs of U_WARM go to scratch
+  A.Q = da.zeros<double>(B * n * n); A.q = da.zeros<double>(B * n); A.gtl = da.zeros<double>(B * n); A.g = da.zeros<double>(B * m);
   return units_launch(game, params, threads, smem_limit_doubles, A, da, plan);
 }
 

@@ -102,17 +102,49 @@ def factor(game, params, H, q, threads=256, smem_limit_doubles=None):
     return out
 
 
-def qp(game, params, x0, u, l, H, q, q2=None, threads=256, smem_limit_doubles=None):
-    """Evaluation at (x0, u, l), a cold QP at (H, q) on its constraints and, with q2, a warm QP at (H, q2)."""
-    x0, u, l, H, q, q2 = (_f64(a) for a in (x0, u, l, H, q, q2))
+def _warm_lists(prev, B):
+    """A list of B warm-start lists (id sequences) as the padded array prev[B, kmax] and the counts kprev[B]."""
+    if prev is None:
+        return None, None, 0
+    assert len(prev) == B
+    kmax = max(1, max(len(p) for p in prev))
+    arr, cnt = np.zeros((B, kmax), np.int32), np.array([len(p) for p in prev], np.int32)
+    for b, p in enumerate(prev):
+        arr[b, :len(p)] = p
+    return arr, cnt, kmax
+
+
+def qp(game, params, x0, u, l, H, q, q2=None, g=None, prev=None, threads=256, smem_limit_doubles=None):
+    """Evaluation at (x0, u, l), a QP at (H, q) on its constraints -- with the offsets g[B, m] in place of the evaluated
+    ones if given; cold, or from the warm-start lists prev (B id sequences) if given -- and, with q2, a warm QP at
+    (H, q2) from the first QP's active set.  it / na: main-loop iterations and active rows at the end."""
+    x0, u, l, H, q, q2, g = (_f64(a) for a in (x0, u, l, H, q, q2, g))
     B, n, m = x0.shape[0], game.n, game.m
+    pv, kp, kmax = _warm_lists(prev, B)
     out = dict(Q=np.zeros((B, n, n)), q=np.zeros((B, n)), gtl=np.zeros((B, n)), g=np.zeros((B, m)),
-               st=np.zeros(B, np.int32), it=np.zeros(B, np.int32), du=np.zeros((B, n)), lam=np.zeros((B, m)),
-               st2=np.zeros(B, np.int32), it2=np.zeros(B, np.int32), du2=np.zeros((B, n)), lam2=np.zeros((B, m)))
+               st=np.zeros(B, np.int32), it=np.zeros(B, np.int32), na=np.zeros(B, np.int32), du=np.zeros((B, n)),
+               lam=np.zeros((B, m)), st2=np.zeros(B, np.int32), it2=np.zeros(B, np.int32), na2=np.zeros(B, np.int32),
+               du2=np.zeros((B, n)), lam2=np.zeros((B, m)))
     out["plan"] = _call("units_qp", game, params, threads, smem_limit_doubles, C.c_int(B), _p(x0), _p(u), _p(l), _p(H),
-                        _p(q), _p(q2), *(_p(out[k]) for k in ("Q", "q", "gtl", "g", "st", "it", "du", "lam", "st2",
-                                                              "it2", "du2", "lam2")))
+                        _p(q), _p(q2), _p(g), _p(pv), _p(kp), C.c_int(kmax),
+                        *(_p(out[k]) for k in ("Q", "q", "gtl", "g", "st", "it", "na", "du", "lam", "st2", "it2", "na2",
+                                               "du2", "lam2")))
     return out
+
+
+def warm_start(game, params, x0, u, l, H, q, g, prev, threads=256, smem_limit_doubles=None):
+    """Evaluation at (x0, u, l) (offsets g[B, m] in place of the evaluated ones if given), qp_factor of H and
+    gi_warm_start from the lists prev: per instance the S-pair the main loop would start from, as "act" (list of ids),
+    "xq" and "lam_act" (array of len(act))."""
+    x0, u, l, H, q, g = (_f64(a) for a in (x0, u, l, H, q, g))
+    B, n = x0.shape[0], game.n
+    pv, kp, kmax = _warm_lists(prev, B)
+    iq, act, xq, lam = np.zeros(B, np.int32), np.zeros((B, n), np.int32), np.zeros((B, n)), np.zeros((B, n))
+    plan = _call("units_warm", game, params, threads, smem_limit_doubles, C.c_int(B), _p(x0), _p(u), _p(l), _p(H), _p(q),
+                 _p(g), _p(pv), _p(kp), C.c_int(kmax), _p(iq), _p(act), _p(xq), _p(lam))
+    assert (iq >= 0).all(), "units_warm: H not positive definite"
+    return dict(act=[act[b, :iq[b]].copy() for b in range(B)], xq=xq,
+                lam_act=[lam[b, :iq[b]].copy() for b in range(B)], plan=plan)
 
 
 def G_products(game, params, x0, u, l, v, w, rows, threads=256, smem_limit_doubles=None):

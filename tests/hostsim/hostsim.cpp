@@ -113,6 +113,53 @@ static int hs_qp_common(HsHandle* h, double* H, const double* q, double* du, dou
   return st;
 }
 int hs_qp(void* hp, double* H, const double* q, double* du, double* lam, int* iters) { return hs_qp_common((HsHandle*)hp, H, q, du, lam, iters, 0); }
+// H into matA, q into a private copy, the offsets g[m] (if given) in place of the evaluated ones and the warm-start list
+// prev[0..k) into Q.act; false if the list is out of range.  The caller restores E.g from gsave.
+static bool hs_qp_inputs(HsHandle* h, const double* H, const double* q, const double* g, const int* prev, int k,
+                         std::vector<double>& qc, std::vector<double>& gsave) {
+  const int n = h->D.n, m = h->D.m;
+  if (k < 0 || k > n || (k > 0 && !prev)) return false;
+  for (int i = 0; i < k; ++i) if (prev[i] < 0 || prev[i] >= m) return false;
+  for (int i = 0; i < n; ++i) memcpy(h->W.B.matA + (size_t)i * h->D.ld, H + (size_t)i * n, sizeof(double) * n);
+  qc.assign(q, q + n);
+  gsave.assign(h->W.E.g, h->W.E.g + m);
+  if (g) memcpy(h->W.E.g, g, sizeof(double) * m);
+  for (int i = 0; i < k; ++i) h->W.Q.act[i] = prev[i];
+  h->W.Q.act[n] = k;
+  return true;
+}
+// QP at the last evaluated point with H (n*n), q and, if given, the offsets g[m] in place of the evaluated ones; from the
+// warm-start list prev[0..k) if k > 0, cold otherwise.  out = {status, main-loop iterations, active rows}
+int hs_qp_g(void* hp, const double* H, const double* q, const double* g, const int* prev, int k, double* du, double* lam,
+            int* out) {
+  HsHandle* h = (HsHandle*)hp; Cta c;
+  std::vector<double> qc, gsave;
+  if (!hs_qp_inputs(h, H, q, g, prev, k, qc, gsave)) return -1;
+  int it = 0, na = 0;
+  out[0] = qp_solve_gi<false>(c, h->D, h->W.E, qc.data(), h->W.Q, h->W.B, &it, &na, k > 0);
+  out[1] = it; out[2] = na;
+  memcpy(du, h->W.Q.xq, sizeof(double) * h->D.n);
+  memcpy(lam, h->W.Q.lam, sizeof(double) * h->D.m);
+  memcpy(h->W.E.g, gsave.data(), sizeof(double) * h->D.m);
+  return 0;
+}
+// qp_factor and gi_warm_start from prev[0..k) (k >= 1) only: returns iq (-1: H not positive definite, -2: bad list) and
+// the S-pair the main loop would start from, act[0..iq), xq[n], lam_act[0..iq)
+int hs_warm_start(void* hp, const double* H, const double* q, const double* g, const int* prev, int k, int* act,
+                  double* xq, double* lam_act) {
+  HsHandle* h = (HsHandle*)hp; Cta c;
+  std::vector<double> qc, gsave;
+  if (k < 1 || !hs_qp_inputs(h, H, q, g, prev, k, qc, gsave)) return -2;
+  int iq = -1;
+  if (qp_factor<false>(c, h->D, qc.data(), h->W.Q, h->W.B)) {
+    iq = gi_warm_start<false>(c, h->D, h->W.E, qc.data(), h->W.Q, h->W.B, k);
+    memcpy(act, h->W.Q.act, sizeof(int) * iq);
+    memcpy(xq, h->W.Q.xq, sizeof(double) * h->D.n);
+    memcpy(lam_act, h->W.Q.lam_act, sizeof(double) * iq);
+  }
+  memcpy(h->W.E.g, gsave.data(), sizeof(double) * h->D.m);
+  return iq;
+}
 int hs_qp_warm(void* hp, double* H, const double* q, double* du, double* lam, int* iters) { return hs_qp_common((HsHandle*)hp, H, q, du, lam, iters, 1); }
 // qp_factor of H (n*n): returns ok; L (lower triangle, zero above), Y = L^-1 (all n x n entries as stored), xq = -H^-1 q
 int hs_factor(void* hp, const double* H, const double* q, double* L, double* Y, double* xq) {

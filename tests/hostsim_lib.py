@@ -42,11 +42,13 @@ def load(asan=False, merge=False, guard=False, fma=False):
     lib.hs_create_v2.restype = C.c_void_p
     lib.hs_create_v2.argtypes = [C.POINTER(gs), C.POINTER(ParamsV2Struct)]
     for name in ["hs_destroy", "hs_dims", "hs_evaluate", "hs_G_dense", "hs_G_times", "hs_GT_times", "hs_nearest_pd",
-                 "hs_qp", "hs_qp_warm", "hs_factor", "hs_plan", "hs_lsqr", "hs_solve"]:
+                 "hs_qp", "hs_qp_warm", "hs_qp_g", "hs_warm_start", "hs_factor", "hs_plan", "hs_lsqr", "hs_solve"]:
         getattr(lib, name).argtypes = None
     lib.hs_nearest_pd.restype = C.c_int
     lib.hs_qp.restype = C.c_int
     lib.hs_qp_warm.restype = C.c_int
+    lib.hs_qp_g.restype = C.c_int
+    lib.hs_warm_start.restype = C.c_int
     lib.hs_factor.restype = C.c_int
     lib.hs_lsqr.restype = C.c_int
     lib.hs_guard_check.restype = C.c_int
@@ -131,6 +133,27 @@ class HostSim:
         it = C.c_int(0)
         st = self.lib.hs_qp_warm(self.h, _p(H), _p(q), _p(du), _p(lam), C.byref(it))
         return st, du, lam, it.value
+
+    def qp_g(self, H, q, g=None, prev=None):
+        """QP at (H, q) on the evaluated constraints with the offsets g in their place (if given), from the warm-start
+        list prev (gi_warm_start) if given, cold otherwise: (status, du, lam, main-loop iterations, active rows)."""
+        H, q, g = (None if a is None else np.ascontiguousarray(a, dtype=np.float64) for a in (H, q, g))
+        prev = np.ascontiguousarray([] if prev is None else prev, dtype=np.int32)
+        du, lam, out = np.zeros(self.n), np.zeros(self.m), np.zeros(3, dtype=np.int32)
+        rc = self.lib.hs_qp_g(self.h, _p(H), _p(q), None if g is None else _p(g), _p(prev), C.c_int(len(prev)), _p(du),
+                              _p(lam), _p(out))
+        assert rc == 0, "hs_qp_g: bad warm-start list"
+        return int(out[0]), du, lam, int(out[1]), int(out[2])
+
+    def warm_start(self, H, q, g, prev):
+        """qp_factor and gi_warm_start only: the S-pair (act, xq, lam_act) the main loop would start from."""
+        H, q, g = (None if a is None else np.ascontiguousarray(a, dtype=np.float64) for a in (H, q, g))
+        prev = np.ascontiguousarray(prev, dtype=np.int32)
+        act, xq, lam_act = np.zeros(self.n, dtype=np.int32), np.zeros(self.n), np.zeros(self.n)
+        iq = self.lib.hs_warm_start(self.h, _p(H), _p(q), None if g is None else _p(g), _p(prev), C.c_int(len(prev)),
+                                    _p(act), _p(xq), _p(lam_act))
+        assert iq >= 0, f"hs_warm_start failed: {iq}"
+        return act[:iq].copy(), xq, lam_act[:iq].copy()
 
     def factor(self, H, q):
         """qp_factor: (ok, L, Y = L^-1 as stored, xq = -H^-1 q)."""
